@@ -4,6 +4,7 @@ dispersion + Wald, with the default norm="combined" theta grid) on synthetic gen
 (BASELINE.json configs[2], the configuration the metric's target is quoted on; it fits one GPU).
 
     python bench.py --gpus N --steps K --warmup W              # this repo's CUDA path
+    python bench.py --gpus 1 --steps K --dump-outputs DIR      # ... and the outputs of the last step as DIR/<name>.npy
     python bench.py --impl reference --gpus N --steps K ...    # CPU restatement of the reference (oracle port)
     python bench.py --sweep                                     # region-count sweep (BASELINE.json configs[4])
 
@@ -30,6 +31,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only; the benchmark leaves it as it found it
 
 
 class stdout_to_stderr:
@@ -302,6 +304,30 @@ def stage_dict(tm):
             "grid_refits": tm[4], "trend_and_mad": tm[5], "size_factors": tm[6]}
 
 
+DUMP_BUDGET = 60 * 2 ** 20          # bytes of per-region arrays in one dump (the whole dump stays under 64 MB)
+
+
+def dump_outputs(path, r, n):
+    """Writes what Engine.region_test returned as path/<name>.npy in float64 (integer columns are exact in float64;
+    a scalar that is None, such as theta without a grid, becomes NaN).  When the per-region arrays of all n regions
+    exceed DUMP_BUDGET, they are cut to the same seeded sample of regions on every run with the same arguments, and
+    the sampled region indices go to region_index.npy."""
+    per_region = {k: v for k, v in r.items()
+                  if isinstance(v, np.ndarray) and v.shape[-1] == n and k not in ("sizeFactors", "deviances")}
+    width = sum(v.size // n for v in per_region.values())
+    m = min(n, DUMP_BUDGET // (8 * (width + 1)))
+    idx = None if m == n else np.sort(np.random.default_rng(20261020).choice(n, m, replace=False))
+    os.makedirs(path, exist_ok=True)
+    for k, v in r.items():
+        if k in per_region:
+            v = v if idx is None else v[..., idx]
+        elif v is None:
+            v = np.nan
+        np.save(os.path.join(path, k + ".npy"), np.asarray(v, dtype=np.float64))
+    if idx is not None:
+        np.save(os.path.join(path, "region_index.npy"), idx.astype(np.float64))
+
+
 def run_strong(R, args, d_full):
     """ONE genome-wide set partitioned by bait over the ranks (the north-star configuration), timed like the main line and
     checked against a single-GPU run of the whole set on rank 0."""
@@ -453,7 +479,7 @@ def run_sweep(R, args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of every timed section")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="cuda", choices=["cuda", "reference"])
     ap.add_argument("--workload", default="c3")
@@ -466,7 +492,14 @@ def main():
                          "bait across the ranks (cd_plan_shards)")
     ap.add_argument("--sweep", action="store_true", help="region-count sweep instead of the bench line")
     ap.add_argument("--sweep-sizes", default=None, help="comma-separated total region counts")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last device-resident step returned (rank 0's regions) as DIR/<name>.npy, float64, "
+                         "at most 64 MB: a fixed seeded sample of the regions when all of them would not fit")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.sweep or args.impl != "cuda"):
+        ap.error("--dump-outputs applies to the bench line of the CUDA path")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -565,19 +598,26 @@ def main():
     fp64 = fp64_roofline(e, d, tm[2], fp64_peak, flop_tab, flop_src)
     fp64["kernel"] = "fit_disp_kernel (dispersion line searches: %.0f %% of the step)" % (100.0 * tm[2] / dev_ms)
 
+    if args.dump_outputs:
+        # the timed step once more on the same resident inputs, its outputs fetched this time.  Its reductions run in a
+        # fixed order (no floating-point atomics), so this is what the last timed step computed.  Collective on all ranks.
+        e.aggregate(fetch=False)
+        r_dump = e.region_test(fetch="all")
+        if rank == 0:
+            dump_outputs(args.dump_outputs, r_dump, n)
+
     # end-to-end steps (host buffers in, table columns out)
     e.set_regions(d.row_off)
-    e2e_steps = max(3, args.steps)
     step_e2e(0, 1)
     step_e2e(0, 1)
-    e2e_dev_ms, e2e_wall_ms, _ = R.timed(step_e2e, e2e_steps)
+    e2e_dev_ms, e2e_wall_ms, _ = R.timed(step_e2e, args.steps)
 
     # the upload alone, all ranks at once: what the host side of this box delivers to N GPUs together (the e2e step cannot
     # be shorter than this; at N = 8 it is what bounds it)
     def step_upload(k, steps):
         upload()
         e.aggregate(fetch=False)
-    up_ms, _, _ = R.timed(step_upload, 3)
+    up_ms, _, _ = R.timed(step_upload, args.steps)
 
     # the same step started one stage earlier: per-replicate CHiCAGO tables -> fused assembly + aggregation
     # (cd_assemble) -> region test.  Reported beside the main line, not instead of it.
@@ -611,10 +651,10 @@ def main():
 
         for _ in range(2):
             step_asm_resident(0, 1)
-        a_dev_ms, _, a_tm = R.timed(step_asm_resident, max(2, args.steps // 2))
+        a_dev_ms, _, a_tm = R.timed(step_asm_resident, args.steps)
         for _ in range(2):
             step_asm_e2e(0, 1)
-        a_e2e_ms, _, _ = R.timed(step_asm_e2e, max(3, args.steps))
+        a_e2e_ms, _, _ = R.timed(step_asm_e2e, args.steps)
         asm = {"what": "per-replicate CHiCAGO tables (s_j, s_i, tblb/tlb, Tmean table, distance function, sparse counts) -> cd_assemble "
                        "(joins + Bmean/Tmean + count merge + region sums in one kernel) -> cd_region_test",
                "ms_per_step": a_dev_ms, "assemble_kernel_ms": a_tm[0], "e2e_ms_per_step": a_e2e_ms, "h2d_bytes_per_step": asm_h2d}
@@ -664,7 +704,7 @@ def main():
                 "roofline": fp64,
                 "roofline_hbm": hbm_roofline(d, tm[0], peaks, peak_src),
                 "e2e": {"value": n_tot / (e2e_dev_ms * 1e-3), "unit": UNIT, "ms_per_step": e2e_dev_ms, "wall_ms_per_step": e2e_wall_ms,
-                        "steps": e2e_steps,
+                        "steps": args.steps,
                         "h2d_bytes_per_step": int(N_host.numel() * 4 + FM_host.numel() * 8),
                         "d2h_bytes_per_step": int(n * (6 * 8 + 1)),
                         "upload_alone": {"what": "cd_set_sample_rows of one batch + cd_aggregate and nothing else, all ranks at "
