@@ -1202,7 +1202,7 @@ constexpr int kScalTrend = 192;       // per fit: 8 doubles (coefficients, statu
 constexpr int kScalSums = 384;        // per fit: S + 1 masked column sums of the normalisation factors
 constexpr int kScalSize = 1024;
 // layout of the pinned host scratch ctx->h_pinned (doubles)
-constexpr int kPinTrend = 0, kPinMad = 128, kPinErr = 144, kPinDev = 160, kPinTrendIn = 200, kPinSf = 400;
+constexpr int kPinTrend = 0, kPinMad = 128, kPinErr = 144, kPinBad = 145, kPinDev = 160, kPinTrendIn = 200, kPinSf = 400;
 
 // R median() of the finite entries of B columns (column c at base + c*stride, n local values each, optionally
 // transformed to |x - center[c]|) over ALL ranks -> out_dev[c] = scale * median (exp'ed if do_exp): one cooperative
@@ -1240,16 +1240,25 @@ int size_factors(cd_ctx* ctx, double* sf_host)
 {
     const int S = ctx->des.S;
     const int64_t n = ctx->n;
+    // counters[7] (zeroed at the start of every cd_region_test) is a double: 1.0 when a count is NA or negative
+    double* bad_dev = reinterpret_cast<double*>(ctx->counters.p + 7);
     CD_CUDA(ctx, ctx->g_LR.ensure((size_t)S * (size_t)n));
-    CD_LAUNCHN(ctx, 1, launch_log_ratios(n, S, ctx->K.p, ctx->g_LR.p, ctx->st));
+    CD_LAUNCHN(ctx, 1, launch_log_ratios(n, S, ctx->K.p, ctx->g_LR.p, bad_dev, ctx->st));
     int rc = medians(ctx, ctx->g_LR.p, n, n, S, nullptr, ctx->scal.p + kScalSf, 1, 1.0);
     if (rc != CD_OK) return rc;
+    // every rank must refuse together, or the clean ones would wait for the others in the next collective
+    CD_COMM(ctx, ctx->comm.allreduce_sum(bad_dev, 1, ctx->st));
     CD_CUDA(ctx, cudaMemcpyAsync(ctx->h_pinned + kPinSf, ctx->scal.p + kScalSf, sizeof(double) * S, cudaMemcpyDeviceToHost, ctx->st));
     CD_CUDA(ctx, cudaMemcpyAsync(ctx->h_pinned + kPinErr, ctx->counters.p + 10, sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->st));
+    CD_CUDA(ctx, cudaMemcpyAsync(ctx->h_pinned + kPinBad, bad_dev, sizeof(double), cudaMemcpyDeviceToHost, ctx->st));
     CD_CUDA(ctx, cudaStreamSynchronize(ctx->st));
     unsigned long long errw;
     memcpy(&errw, ctx->h_pinned + kPinErr, sizeof(errw));
     if ((rc = check_peer_exchange(ctx, errw)) != CD_OK) return rc;
+    if (ctx->h_pinned[kPinBad] != 0.0)
+        return ctx->fail(CD_EINVAL, "NA or negative values in the count matrix (DESeq2: \"NA values are not allowed in the count "
+                                    "matrix\" / \"some values in assay are negative\"); NA_integer_ marks a region sum beyond "
+                                    "the int32 range");
     for (int s = 0; s < S; s++) {
         sf_host[s] = ctx->h_pinned[kPinSf + s];
         if (std::isnan(sf_host[s]))
@@ -1548,7 +1557,7 @@ int cd_region_test(cd_ctx* ctx, const cd_options* opt, cd_results* out)
 
     CD_CUDA(ctx, ctx->eval_counts.ensure(16));
     CD_CUDA(ctx, cudaMemsetAsync(ctx->eval_counts.p, 0, 16 * sizeof(unsigned long long), st));
-    CD_CUDA(ctx, cudaMemsetAsync(ctx->counters.p + 4, 0, 3 * sizeof(unsigned long long), st));
+    CD_CUDA(ctx, cudaMemsetAsync(ctx->counters.p + 4, 0, 4 * sizeof(unsigned long long), st));     // [4..6] waits, [7] bad counts
     ctx->n_eval_calls = 0;
     ctx->trend_passes = 0;
     CD_CUDA(ctx, cudaEventRecord(ctx->ev[2], st));

@@ -83,7 +83,8 @@ cudaError_t tb_launch_count_gather(int64_t m_valid, const unsigned long long* so
                                    const int32_t* N_rows, int32_t* cnt_oe, int32_t* cnt_N, cudaStream_t st);
 
 // ---- size factors + stage 2: offsets (chicdiff.R:1561-1562, 1583-1589, 1635-1638) ------
-cudaError_t launch_log_ratios(int64_t n, int S, const int32_t* K, double* LR /*S x n, +inf = excluded*/,
+// bad (one double, zeroed by the caller) is set to 1.0 when any count is negative (NA_integer_ included)
+cudaError_t launch_log_ratios(int64_t n, int S, const int32_t* K, double* LR /*S x n, +inf = excluded*/, double* bad,
                               cudaStream_t st);
 // nf (S x G*n) for the G fits of a batch (mode 2: fit g at theta.v[g]); Kb != null also replicates K (S x n) into the
 // batch layout (S x G*n)

@@ -128,29 +128,33 @@ cudaError_t launch_xim(int G, int S, const double* sums, double* xim, cudaStream
 
 // ---------------------------------------------------------------------------------------
 // size factors: LR[s][i] = log K[s][i] - mean_s' log K[s'][i] for rows with every K > 0,
-// +inf otherwise (excluded from the medians)
+// +inf otherwise (excluded from the medians).  This is the one pass of a region test that reads every count, so it
+// also checks them: DESeqDataSetFromMatrix (chicdiff.R:1556-1559) refuses NA (NA_integer_ = INT32_MIN, what the
+// aggregation writes for a sum beyond the int32 range) and negative counts; *bad = 1.0 tells the host to do the same.
 // ---------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
-log_ratios_kernel(int64_t n, int S, const int32_t* __restrict__ K, double* __restrict__ LR)
+log_ratios_kernel(int64_t n, int S, const int32_t* __restrict__ K, double* __restrict__ LR, double* __restrict__ bad)
 {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     double acc = 0.0;
-    bool ok = true;
+    bool ok = true, neg = false;
     for (int s = 0; s < S; s++) {
         const int32_t k = K[(int64_t)s * n + i];
         ok = ok && (k > 0);
+        neg = neg || (k < 0);
         acc += log((double)k);
     }
+    if (neg) *bad = 1.0;                       // every writer stores the same value: no atomic needed
     const double lgm = acc / S;
     for (int s = 0; s < S; s++)
         LR[(int64_t)s * n + i] = ok ? log((double)K[(int64_t)s * n + i]) - lgm : INFINITY;
 }
 
-cudaError_t launch_log_ratios(int64_t n, int S, const int32_t* K, double* LR, cudaStream_t st)
+cudaError_t launch_log_ratios(int64_t n, int S, const int32_t* K, double* LR, double* bad, cudaStream_t st)
 {
     if (n == 0) return cudaSuccess;
-    log_ratios_kernel<<<blocks_for(n, 256), 256, 0, st>>>(n, S, K, LR);
+    log_ratios_kernel<<<blocks_for(n, 256), 256, 0, st>>>(n, S, K, LR, bad);
     return cudaGetLastError();
 }
 

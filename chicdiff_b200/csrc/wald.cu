@@ -140,7 +140,7 @@ template <int P>
 __global__ void __launch_bounds__(kWaldThreads)
 wald_irls_kernel(int64_t n, int S, const CdDesign* __restrict__ des, const int32_t* __restrict__ K, const double* __restrict__ nf,
                  const double* __restrict__ dispersion, const uint8_t* __restrict__ flags,
-                 const double* __restrict__ cmat, const double* __restrict__ beta0,
+                 const double* __restrict__ cmat, double* __restrict__ beta0,
                  double* __restrict__ beta_out /*P x n, natural log scale*/, int32_t* __restrict__ iter_out,
                  unsigned long long* __restrict__ work_counter)
 {
@@ -160,12 +160,12 @@ wald_irls_kernel(int64_t n, int S, const CdDesign* __restrict__ des, const int32
 
     bool active = false, exhausted = false, fresh = false;
     int64_t i = 0;
-    double beta[P], rhs[P];
+    double beta[P], beta_mu[P], rhs[P];          // beta_mu: the coefficients of the last sweep (of the fitted means)
     Sym<P> A;
     double alpha = 1.0, size = 1.0, dev_old = 0.0;
     int iter = 0;
 #pragma unroll
-    for (int u = 0; u < P; u++) { beta[u] = 0.0; rhs[u] = 0.0; }
+    for (int u = 0; u < P; u++) { beta[u] = 0.0; beta_mu[u] = 0.0; rhs[u] = 0.0; }
 #pragma unroll
     for (int k = 0; k < P * (P + 1) / 2; k++) A.v[k] = 0.0;
 
@@ -224,7 +224,11 @@ wald_irls_kernel(int64_t n, int S, const CdDesign* __restrict__ des, const int32
         __syncwarp();
         // ---- one sweep over the replicates at the current coefficients ----
         double dev = 0.0;
-        if (active && !finished) irls_pass<P>(beta, alpha, size, S, stride, ys, nfs, cs, Xs, tabh, A, rhs, dev);
+        if (active && !finished) {
+            irls_pass<P>(beta, alpha, size, S, stride, ys, nfs, cs, Xs, tabh, A, rhs, dev);
+#pragma unroll
+            for (int u = 0; u < P; u++) beta_mu[u] = beta[u];
+        }
         __syncwarp();
         if (active && !finished) {
             if (fresh) {
@@ -240,6 +244,11 @@ wald_irls_kernel(int64_t n, int S, const CdDesign* __restrict__ des, const int32
         if (finished) {
 #pragma unroll
             for (int u = 0; u < P; u++) beta_out[(int64_t)u * n + i] = beta[u];
+            // DESeq2's fitBeta stops on |beta| > 30 before it updates the fitted means, and its weights for the standard
+            // errors and hat values are those means: the finalisation takes them from here (this row's start values
+            // are not read again)
+#pragma unroll
+            for (int u = 0; u < P; u++) beta0[(int64_t)u * n + i] = beta_mu[u];
             iter_out[i] = iter;
             active = false;
         }
@@ -271,7 +280,7 @@ __global__ void __launch_bounds__(kWaldThreads)
 wald_final_kernel(int64_t n, int S, const CdDesign* __restrict__ des, const int32_t* __restrict__ K, const double* __restrict__ nf,
                   const double* __restrict__ dispersion, uint8_t* __restrict__ flags,
                   const double* __restrict__ cmat, const double* __restrict__ beta_nat,
-                  const int32_t* __restrict__ iter_in,
+                  const double* __restrict__ beta_mu_in, const int32_t* __restrict__ iter_in,
                   double* __restrict__ beta_out, double* __restrict__ se_out, double* __restrict__ stat_out,
                   double* __restrict__ pvalue_out, double* __restrict__ deviance_out, double* __restrict__ maxCooks_out,
                   int32_t* __restrict__ betaIter_out, double* __restrict__ mu_out)
@@ -298,15 +307,16 @@ wald_final_kernel(int64_t n, int S, const CdDesign* __restrict__ des, const int3
     const double alpha = dispersion[i];
     const double size = rcp_pos(alpha);
     const double lambda = 1e-6 / (kLn2 * kLn2);
-    double beta[P], se[P];
+    double beta[P], beta_w[P], se[P];       // beta_w: the coefficients of the fitted means that weigh X'WX and the hat values
     int iter = 1;
     double qsum = 0.0;
     for (int j = 0; j < S; j++) qsum += (double)K[(int64_t)j * n + i] * rcp_pos(nf[(int64_t)j * n + i]);
     if (P == 1) {
         beta[0] = log_pos(qsum / S);          // fitNbinomGLMs intercept-only shortcut (natural log scale)
+        beta_w[0] = beta[0];
     } else {
 #pragma unroll
-        for (int u = 0; u < P; u++) beta[u] = beta_nat[(int64_t)u * n + i];
+        for (int u = 0; u < P; u++) { beta[u] = beta_nat[(int64_t)u * n + i]; beta_w[u] = beta_mu_in[(int64_t)u * n + i]; }
         iter = iter_in[i];
     }
     if (mu_only) {
@@ -325,12 +335,12 @@ wald_final_kernel(int64_t n, int S, const CdDesign* __restrict__ des, const int3
     double loglike = 0.0;
     for (int j = 0; j < S; j++) {
         const double yj = (double)K[(int64_t)j * n + i], nfj = nf[(int64_t)j * n + i];
-        double eta = 0.0;
+        double eta = 0.0, eta_w = 0.0;
 #pragma unroll
-        for (int u = 0; u < P; u++) eta += Xs[j * P + u] * beta[u];
+        for (int u = 0; u < P; u++) { eta += Xs[j * P + u] * beta[u]; eta_w += Xs[j * P + u] * beta_w[u]; }
         const double muw = nfj * exp(eta);                   // unfloored, as stored by nbinomWaldTest
         loglike += nb_logdens(yj, size, alpha, muw, cmat[(int64_t)j * n + i], tabh);
-        const double muc = (P == 1) ? muw : fmax(muw, kMinMu);
+        const double muc = (P == 1) ? muw : fmax(nfj * exp(eta_w), kMinMu);
         const double w = muc * rcp_pos(1.0 + alpha * muc);
 #pragma unroll
         for (int u = 0; u < P; u++)
@@ -389,11 +399,11 @@ wald_final_kernel(int64_t n, int S, const CdDesign* __restrict__ des, const int3
         double mc = -INFINITY, ck_best = -INFINITY, y_best = 0.0;
         for (int j = 0; j < S; j++) {
             const double yj = (double)K[(int64_t)j * n + i], nfj = nf[(int64_t)j * n + i];
-            double eta = 0.0;
+            double eta = 0.0, eta_w = 0.0;
 #pragma unroll
-            for (int u = 0; u < P; u++) eta += Xs[j * P + u] * beta[u];
+            for (int u = 0; u < P; u++) { eta += Xs[j * P + u] * beta[u]; eta_w += Xs[j * P + u] * beta_w[u]; }
             const double muw = nfj * exp(eta);
-            const double muc = (P == 1) ? muw : fmax(muw, kMinMu);
+            const double muc = (P == 1) ? muw : fmax(nfj * exp(eta_w), kMinMu);
             const double w = muc / (1.0 + alpha * muc);
             double h = 0.0;
 #pragma unroll
@@ -511,7 +521,7 @@ cudaError_t launch_wald(int64_t n, int S, int p, const CdDesign* des, const int3
     }
 #define CD_FINAL(P_)                                                                                             \
     wald_final_kernel<P_><<<blocks_for(n, threads), threads, 0, st>>>(n, S, des, K, nf, dispersion, flags, ws.cmat, \
-        ws.beta_nat, ws.iter, beta, betaSE, stat, pvalue, deviance, maxCooks, betaIter, mu_out)
+        ws.beta_nat, ws.beta0, ws.iter, beta, betaSE, stat, pvalue, deviance, maxCooks, betaIter, mu_out)
     switch (p) {
         case 1: CD_FINAL(1); break;
         case 2: CD_IRLS(2); CD_FINAL(2); break;

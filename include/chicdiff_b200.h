@@ -255,7 +255,8 @@ typedef struct {
     int64_t n_nonzero, n_gene_grid, n_map_grid, n_beta_noconv;
 } cd_results;
 
-/* DESeq2Wrap numerics on the aggregated matrices of this context (this rank's shard) */
+/* DESeq2Wrap numerics on the aggregated matrices of this context (this rank's shard).  CD_EINVAL when a count is NA
+ * (INT32_MIN) or negative, on every rank of a sharded run (DESeqDataSetFromMatrix, chicdiff.R:1556-1559). */
 int cd_region_test(cd_ctx* ctx, const cd_options* opt, cd_results* out);
 
 /* ---- several GPUs from ONE process ------------------------------------------------------ */

@@ -338,8 +338,18 @@ static double median_inplace(double* v, int64_t m)
     return (m & 1) ? v[m / 2] : 0.5 * (v[m / 2 - 1] + v[m / 2]);
 }
 
+/* DESeqDataSetFromMatrix (chicdiff.R:1556-1559) refuses NA (NA_integer_ = INT32_MIN) and negative counts */
+static int any_negative(int64_t n, int S, const int32_t* K)
+{
+    for (int64_t j = 0; j < (int64_t)S * n; j++)
+        if (K[j] < 0) return 1;
+    return 0;
+}
+
+/* returns -1 when every region has a zero count, -2 for NA or negative counts */
 int orc_size_factors(int64_t n, int S, const int32_t* K, double* sf)
 {
+    if (any_negative(n, S, K)) return -2;
     double* lgm = (double*)malloc(sizeof(double) * (size_t)n);
     double* buf = (double*)malloc(sizeof(double) * (size_t)n);
     int64_t nfinite = 0;
@@ -855,6 +865,7 @@ int orc_deseq_ex(int64_t n, int S, int p, const double* X, const int32_t* K, con
     const int maxit = 100;
     const double maxDisp = fmax(10.0, (double)S);
     if (S > ORC_MAXS || p > ORC_MAXP || S <= p) return -1;
+    if (any_negative(n, S, K)) return -4;
     design_t d;
     design_init(&d, S, p, X);
 #ifdef _OPENMP

@@ -78,11 +78,16 @@ def aggregate(row_off, N_rows, FM_rows):
     return K, FM
 
 
+NEGATIVE_COUNTS = "NA or negative values in the count matrix"
+
+
 def size_factors(K):
     K = np.ascontiguousarray(K, dtype=np.int32)
     S, n = K.shape
     sf = np.empty(S, np.float64)
     rc = lib().orc_size_factors(C.c_int64(n), C.c_int(S), _p(K), _p(sf))
+    if rc == -2:
+        raise ValueError(NEGATIVE_COUNTS)
     if rc != 0:
         raise ValueError("every gene contains at least one zero, cannot compute log geometric means")
     return sf
@@ -141,14 +146,16 @@ def deseq(K, nf, X, prior_var=float("nan"), grid_n=20, nthreads=0, trend=None, v
                lp_evals=sc[8], dlp_evals=sc[9], irls_iters=sc[10], sum_deviance=sc[11], n_nonzero=sc[12])
     if rc != 0:
         raise RuntimeError({-1: "bad design (S<=p or too large)", -2: "S-p<=3 needs dispPriorVar (Monte-Carlo path not restated)",
-                            -3: "parametric dispersion trend failed (local fit not restated)"}.get(rc, "rc=%d" % rc))
+                            -3: "parametric dispersion trend failed (local fit not restated)",
+                            -4: NEGATIVE_COUNTS}.get(rc, "rc=%d" % rc))
     return res
 
 
 def region_test(K, FMagg, X, norm="combined", theta=None, theta_grid=(0, .25, .5, .75, 1), prior_var=float("nan"),
-                prior_var_grid=float("nan"), nthreads=0, trend=None, var_log_disp=None, margins=False, L=None):
+                prior_var_grid=float("nan"), nthreads=0, trend=None, var_log_disp=None, margins=False, L=None, grid_n=20):
     """DESeq2Wrap numerics (chicdiff.R:1551-1674): size factors, offsets, theta grid, final fit.
-    trend / var_log_disp / margins / L apply to the final fit only (see deseq)."""
+    trend / var_log_disp / margins / L apply to the final fit only (see deseq); grid_n (fitDispGrid length) to every fit.
+    NA (INT32_MIN) or negative counts raise ValueError, as DESeqDataSetFromMatrix stops on them."""
     S, n = K.shape
     sf = size_factors(K)
     out = {"sizeFactors": sf, "deviances": None}
@@ -162,7 +169,7 @@ def region_test(K, FMagg, X, norm="combined", theta=None, theta_grid=(0, .25, .5
         X1 = np.ones((S, 1))
         for tt in theta_grid:
             nf = norm_factors(FMagg, sf, "combined", tt)
-            r = deseq(K, nf, X1, prior_var=prior_var_grid, nthreads=nthreads)
+            r = deseq(K, nf, X1, prior_var=prior_var_grid, grid_n=grid_n, nthreads=nthreads)
             devs.append(r["sum_deviance"])
         devs = np.asarray(devs)
         out["deviances"] = devs
@@ -176,7 +183,7 @@ def region_test(K, FMagg, X, norm="combined", theta=None, theta_grid=(0, .25, .5
     out["theta"] = theta if norm == "combined" else None
     nf = norm_factors(FMagg, sf, norm, 0.0 if theta is None else theta)
     out["nf"] = nf
-    out.update(deseq(K, nf, X, prior_var=prior_var, nthreads=nthreads, trend=trend, var_log_disp=var_log_disp,
+    out.update(deseq(K, nf, X, prior_var=prior_var, grid_n=grid_n, nthreads=nthreads, trend=trend, var_log_disp=var_log_disp,
                      margins=margins, L=L))
     return out
 

@@ -104,6 +104,28 @@ def test_aggregate_edge_cases():
     assert FM[0, 0] == 0.0 and FM[0, 1] == 0.5 and np.isnan(FM[0, 2]) and FM[0, 3] == 2.0
 
 
+def test_na_and_negative_counts_are_refused(tiny):
+    """DESeqDataSetFromMatrix (chicdiff.R:1556-1559) stops on NA and negative counts; so does the oracle, whether the NA
+    comes from a region sum beyond the int32 range (NA_integer_ = INT32_MIN) or the counts are handed over as they are"""
+    import parity
+    X, row_off, N, FMr = parity.aggregate_edge_rows()
+    K, FM = O.aggregate(row_off, N, FMr)
+    assert K[2, 6] == -2147483648
+    with pytest.raises(ValueError, match=O.NEGATIVE_COUNTS):
+        O.region_test(K, FM, X)
+    d, K, FM = tiny
+    O.region_test(K, FM, d.X, theta=0.5)                                   # the clean matrix runs
+    for v in (-1, -3, -2147483648):
+        Kb = K.copy()
+        Kb[2, 5] = v
+        with pytest.raises(ValueError, match=O.NEGATIVE_COUNTS):
+            O.size_factors(Kb)
+        with pytest.raises(ValueError, match=O.NEGATIVE_COUNTS):
+            O.region_test(Kb, FM, d.X, theta=0.5)
+        with pytest.raises(RuntimeError, match=O.NEGATIVE_COUNTS):
+            O.deseq(Kb, np.ones(Kb.shape), d.X, prior_var=1.0)
+
+
 def test_size_factors_against_numpy(tiny):
     d, K, FM = tiny
     sf = O.size_factors(K)
