@@ -8,6 +8,7 @@
 #include "comm.h"
 #include "results_host.h"
 #include <algorithm>
+#include <climits>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -249,6 +250,8 @@ struct cd_ctx {
     DevBuf<unsigned int> res_idx[2], res_cnt;
     DevBuf<double> res_pv, res_padj, res_bms, res_ps, res_smalld, res_cmin, res_smin;
     DevBuf<unsigned char> res_tmp;
+    DevBuf<double> res_in;                               // cd_results_device: uploaded columns
+    DevBuf<uint8_t> res_in_flags;
     // columns of the last cd_parse_chinput
     int64_t ch_rows = 0;
     DevBuf<int32_t> ch_bait, ch_oe, ch_N, ch_len;
@@ -1642,17 +1645,12 @@ int cd_region_test(cd_ctx* ctx, const cd_options* opt, cd_results* out)
     return CD_OK;
 }
 
-int cd_results_resident(cd_ctx* ctx, double* pvalue_out, double* padj_out, double* scalars_out)
+// results() (Cook's cutoff, independent filtering, BH) on n rows whose columns are in device memory on ctx's device:
+// the body of cd_results_resident (the arrays of the last cd_region_test) and of cd_results_device (uploaded columns)
+static int results_on_device(cd_ctx* ctx, int64_t n, int S, int p, const double* baseMean, const double* maxCooks,
+                             const uint8_t* flags, const double* pvalue, double* pvalue_out, double* padj_out, double* scalars_out)
 {
-    if (!ctx) return CD_EINVAL;
-    if (!ctx->have_results) return ctx->fail(CD_EINVAL, "cd_results_resident: no successful cd_region_test on this context yet");
-    if (ctx->comm.active() && ctx->comm.nranks > 1)
-        return ctx->fail(CD_EINVAL, "cd_results_resident: results() is global over all regions; in a sharded run gather the "
-                                    "columns and call cd_results_adjust");
-    CD_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->st;
-    const int64_t n = ctx->n;
-    const int S = ctx->des.S, p = ctx->des.p;
     const double alpha = 0.1;
     const double cutoff = res_qf(0.99, (double)p, (double)(S - p));
     const size_t nn = (size_t)std::max<int64_t>(n, 1);
@@ -1672,14 +1670,13 @@ int cd_results_resident(cd_ctx* ctx, double* pvalue_out, double* padj_out, doubl
     double* theta = ctx->res_smalld.p + 50;
     unsigned long long *pkey0 = ctx->res_key[0].p, *pkey1 = ctx->res_key[1].p, *bmkey0 = ctx->res_key[2].p, *bmkey1 = ctx->res_key[3].p;
     unsigned int *idx0 = ctx->res_idx[0].p, *idx1 = ctx->res_idx[1].p;
-    const double* baseMean = ctx->g_baseMean.p + ctx->g_off;
-    const uint8_t* flags = ctx->g_flags.p + ctx->g_off;
 
-    CD_LAUNCHN(ctx, 1, res_launch_keys(n, p, cutoff, baseMean, ctx->maxCooks.p, flags, ctx->pvalue.p, ctx->res_pv.p, ctx->res_padj.p,
+    CD_LAUNCHN(ctx, 1, res_launch_keys(n, p, cutoff, baseMean, maxCooks, flags, pvalue, ctx->res_pv.p, ctx->res_padj.p,
                                        pkey0, bmkey0, idx0, counts, st));
     int j = 0;
     double cut_h[50], theta_h[50];
-    for (int k = 0; k < 50; k++) { cut_h[k] = NAN; theta_h[k] = NAN; }
+    // no rows: the host routine's values (lower = 0, upper = .95, every cut NaN)
+    for (int k = 0; k < 50; k++) { cut_h[k] = NAN; theta_h[k] = (k == 49) ? .95 : 0.0 + k * ((.95 - 0.0) / 49); }
     if (n > 0) {
         size_t bytes = 0;
         CD_CUDA(ctx, cp_sort_pairs_u64(nullptr, bytes, bmkey0, bmkey1, idx0, idx1, n, st));
@@ -1707,6 +1704,42 @@ int cd_results_resident(cd_ctx* ctx, double* pvalue_out, double* padj_out, doubl
         scalars_out[0] = cutoff; scalars_out[1] = cut_h[j]; scalars_out[2] = theta_h[j]; scalars_out[3] = (double)(j + 1);
     }
     return CD_OK;
+}
+
+int cd_results_resident(cd_ctx* ctx, double* pvalue_out, double* padj_out, double* scalars_out)
+{
+    if (!ctx) return CD_EINVAL;
+    if (!ctx->have_results) return ctx->fail(CD_EINVAL, "cd_results_resident: no successful cd_region_test on this context yet");
+    if (ctx->comm.active() && ctx->comm.nranks > 1)
+        return ctx->fail(CD_EINVAL, "cd_results_resident: results() is global over all regions; in a sharded run gather the "
+                                    "columns and call cd_results_device or cd_results_adjust");
+    CD_CUDA(ctx, cudaSetDevice(ctx->device));
+    return results_on_device(ctx, ctx->n, ctx->des.S, ctx->des.p, ctx->g_baseMean.p + ctx->g_off, ctx->maxCooks.p,
+                             ctx->g_flags.p + ctx->g_off, ctx->pvalue.p, pvalue_out, padj_out, scalars_out);
+}
+
+int cd_results_device(cd_ctx* ctx, int64_t n, int S, int p, const double* baseMean, const double* maxCooks, const uint8_t* flags,
+                      const double* pvalue, double* pvalue_out, double* padj_out, double* scalars_out)
+{
+    if (!ctx) return CD_EINVAL;
+    if (n < 0 || n > (int64_t)INT_MAX || S <= p || p < 1 || (n > 0 && (!baseMean || !pvalue)))
+        return ctx->fail(CD_EINVAL, "cd_results_device: bad arguments");
+    CD_CUDA(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->st;
+    const size_t nn = (size_t)std::max<int64_t>(n, 1), bytes = sizeof(double) * (size_t)n;
+    CD_CUDA(ctx, ctx->res_in.ensure(3 * nn));                // baseMean, maxCooks, pvalue
+    CD_CUDA(ctx, ctx->res_in_flags.ensure(nn));
+    double *bm = ctx->res_in.p, *mc = ctx->res_in.p + nn, *pv = ctx->res_in.p + 2 * nn;
+    if (n > 0) {
+        CD_CUDA(ctx, cudaMemcpyAsync(bm, baseMean, bytes, cudaMemcpyHostToDevice, st));
+        CD_CUDA(ctx, cudaMemcpyAsync(pv, pvalue, bytes, cudaMemcpyHostToDevice, st));
+        // no maxCooks: all NaN (0xff bytes), which is never an outlier; no flags: none kept
+        if (maxCooks) CD_CUDA(ctx, cudaMemcpyAsync(mc, maxCooks, bytes, cudaMemcpyHostToDevice, st));
+        else CD_CUDA(ctx, cudaMemsetAsync(mc, 0xff, bytes, st));
+        if (flags) CD_CUDA(ctx, cudaMemcpyAsync(ctx->res_in_flags.p, flags, (size_t)n, cudaMemcpyHostToDevice, st));
+        else CD_CUDA(ctx, cudaMemsetAsync(ctx->res_in_flags.p, 0, (size_t)n, st));
+    }
+    return results_on_device(ctx, n, S, p, bm, mc, ctx->res_in_flags.p, pv, pvalue_out, padj_out, scalars_out);
 }
 
 int cd_get_dims(const cd_ctx* ctx, int64_t* n, int* S, int* p, int64_t* R)

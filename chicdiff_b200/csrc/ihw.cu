@@ -108,7 +108,8 @@ ihw_bh_write_kernel(int64_t n, const unsigned int* __restrict__ idx_sorted, cons
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= n) return;
     const int64_t m = (int64_t)*n_ok;
-    padj[idx_sorted[t]] = (t < m) ? fmin(1.0, cummin[t]) : NAN;
+    // p.adjust returns a lone non-NA p-value unchanged, above 1 included
+    padj[idx_sorted[t]] = (t < m) ? (m > 1 ? fmin(1.0, cummin[t]) : cummin[t]) : NAN;
 }
 
 struct Scratch {

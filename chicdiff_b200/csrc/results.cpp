@@ -193,7 +193,7 @@ extern "C" int cd_results_adjust(int64_t n, int S, int p, const double* baseMean
     // independent filtering
     int64_t nzero = 0;
     for (int64_t i = 0; i < n; i++) nzero += (baseMean[i] == 0.0);
-    const double lower = n > 0 ? (double)nzero / (double)n : 0.0;
+    const double lower = n > 0 ? cd::res_mean_of_count((uint64_t)nzero, (uint64_t)n) : 0.0;
     const double upper = lower < .95 ? .95 : 1.0;
     const int NT = 50;
     std::vector<double> theta(NT), cut(NT);
@@ -202,13 +202,9 @@ extern "C" int cd_results_adjust(int64_t n, int S, int p, const double* baseMean
     std::sort(fs.begin(), fs.end());
     for (int k = 0; k < NT; k++) {
         if (n == 0) { cut[k] = NAN; continue; }
-        const double index = (double)(n - 1) * theta[k];             // 0-based version of 1 + (n-1) p
-        const int64_t lo = (int64_t)std::floor(index), hi = (int64_t)std::ceil(index);
-        double q = fs[lo];
-        if (index > (double)lo && fs[hi] != q) {
-            const double h = index - (double)lo;
-            q = (1.0 - h) * q + h * fs[hi];
-        }
+        const cd::ResQuantileIndex ix = cd::res_quantile7_index(n, theta[k]);
+        double q = fs[ix.lo];
+        if (ix.h > 0.0 && fs[ix.hi] != q) q = (1.0 - ix.h) * q + ix.h * fs[ix.hi];
         cut[k] = q;
     }
     // rows with a p-value, ascending by p (stable, so ties keep row order like R's order()); the sorted records
@@ -320,12 +316,14 @@ extern "C" int cd_ihw_apply(int64_t n, const double* avDist, const double* pvalu
         ord.reserve((size_t)n);
         for (int64_t i = 0; i < n; i++) { weighted_padj_out[i] = NAN; if (!std::isnan(wp[(size_t)i])) ord.push_back(i); }
         std::stable_sort(ord.begin(), ord.end(), [&](int64_t a, int64_t b) { return wp[(size_t)a] < wp[(size_t)b]; });
+        // p.adjust returns p unchanged when at most one is not NA (`if (n <= 1) return(p0)`): a single weighted p-value
+        // above 1 stays above 1
         const int64_t m = (int64_t)ord.size();
         double running = INFINITY;
         for (int64_t r = m; r >= 1; r--) {
             const int64_t i = ord[(size_t)r - 1];
             running = std::min(running, (double)m / (double)r * wp[(size_t)i]);
-            weighted_padj_out[i] = std::min(1.0, running);
+            weighted_padj_out[i] = m > 1 ? std::min(1.0, running) : running;
         }
     }
     return CD_OK;

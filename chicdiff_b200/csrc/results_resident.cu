@@ -8,6 +8,7 @@
 // which every cut-off is a prefix count over the p-sorted rows.  Chunks of 2048 sorted rows per CTA; the 50
 // cut-offs share one load of the chunk.
 #include "kernels.h"
+#include "results_host.h"
 
 namespace cd {
 
@@ -61,27 +62,24 @@ res_keys_kernel(int64_t n, int p, double cutoff, const double* __restrict__ base
     }
 }
 
-// quantile(baseMean, theta, type 7) for the 50 theta of genefilter's filtered_p call inside results()
+// quantile(baseMean, theta, type 7) for the 50 theta of genefilter's filtered_p call inside results(); lower and the
+// index as R computes them (results_host.h)
 __global__ void res_cutoffs_kernel(int64_t n, const unsigned long long* __restrict__ bm_sorted_keys,
                                    const unsigned long long* __restrict__ counts, double* __restrict__ cut /*50*/,
                                    double* __restrict__ theta_out /*50*/)
 {
     const int k = threadIdx.x;
     if (k >= kNT) return;
-    const double lower = n > 0 ? (double)counts[1] / (double)n : 0.0;
+    const double lower = n > 0 ? res_mean_of_count(counts[1], (uint64_t)n) : 0.0;
     const double upper = lower < .95 ? .95 : 1.0;
     const double step = __ddiv_rn(__dsub_rn(upper, lower), (double)(kNT - 1));
     const double theta = (k == kNT - 1) ? upper : __dadd_rn(lower, __dmul_rn((double)k, step));
     theta_out[k] = theta;
     if (n == 0) { cut[k] = NAN; return; }
-    const double index = __dmul_rn((double)(n - 1), theta);
-    const int64_t lo = (int64_t)floor(index), hi = (int64_t)ceil(index);
-    double q = res_value(bm_sorted_keys[lo]);
-    const double qh = res_value(bm_sorted_keys[hi]);
-    if (index > (double)lo && qh != q) {
-        const double h = __dsub_rn(index, (double)lo);
-        q = __dadd_rn(__dmul_rn(__dsub_rn(1.0, h), q), __dmul_rn(h, qh));
-    }
+    const ResQuantileIndex ix = res_quantile7_index(n, theta);
+    double q = res_value(bm_sorted_keys[ix.lo]);
+    const double qh = res_value(bm_sorted_keys[ix.hi]);
+    if (ix.h > 0.0 && qh != q) q = __dadd_rn(__dmul_rn(__dsub_rn(1.0, ix.h), q), __dmul_rn(ix.h, qh));
     cut[k] = q;
 }
 

@@ -17,7 +17,7 @@ CD_NORM = {"standard": 0, "fullmean": 1, "combined": 2}
 FLAG_ALLZERO, FLAG_GENE_GRID, FLAG_MAP_GRID, FLAG_BETA_NOCONV, FLAG_OUTLIER, FLAG_GENE_NOINCREASE, FLAG_COOKS_KEEP = \
     1, 2, 4, 8, 16, 32, 64
 
-EXPORTED = ["cd_version", "cd_create", "cd_destroy", "cd_last_error", "cd_comm_unique_id", "cd_comm_init", "cd_comm_info", "cd_results_resident", "cd_ihw_apply",
+EXPORTED = ["cd_version", "cd_create", "cd_destroy", "cd_last_error", "cd_comm_unique_id", "cd_comm_init", "cd_comm_info", "cd_results_resident", "cd_results_device", "cd_ihw_apply",
             "cd_plan_shards", "cd_set_design", "cd_set_regions", "cd_set_sample_rows", "cd_set_rows_device",
             "cd_set_aggregated", "cd_aggregate", "cd_region_test", "cd_results_adjust", "cd_launch_count",
             "cd_device_buffers", "cd_last_timings", "cd_last_search_counts", "cd_get_dims", "cd_last_rendezvous", "cd_ihw_apply_device",
@@ -247,6 +247,22 @@ class Engine:
         n = self.n
         pv, padj, sc = np.empty(n), np.empty(n), np.zeros(4)
         self._check(self._L.cd_results_resident(self._h, pv.ctypes.data, padj.ctypes.data, sc.ctypes.data))
+        return dict(pvalue=pv, padj=padj, cooksCutoff=sc[0], filterThreshold=sc[1], filterTheta=sc[2], filterIndex=int(sc[3]))
+
+    def results_device(self, baseMean, maxCooks, flags, pvalue, S, p):
+        """results() on the given columns with the device routine of results_resident() (cd_results_device); arguments
+        and keys as results_adjust().  The columns are copied to this context's GPU; pvalue is not modified."""
+        baseMean = np.ascontiguousarray(baseMean, dtype=np.float64)
+        n = len(baseMean)
+        pvalue = np.ascontiguousarray(pvalue, dtype=np.float64)
+        mc = None if maxCooks is None else np.ascontiguousarray(maxCooks, dtype=np.float64)
+        fl = None if flags is None else np.ascontiguousarray(flags, dtype=np.uint8)
+        if len(pvalue) != n or (mc is not None and len(mc) != n) or (fl is not None and len(fl) != n):
+            raise ValueError("results_device: columns of different lengths")
+        pv, padj, sc = np.empty(n), np.empty(n), np.zeros(4)
+        self._L.cd_results_device.argtypes = [C.c_void_p, C.c_int64, C.c_int, C.c_int] + [C.c_void_p] * 7
+        self._check(self._L.cd_results_device(self._h, n, S, p, _ptr(baseMean), _ptr(mc), _ptr(fl), _ptr(pvalue), _ptr(pv),
+                                               _ptr(padj), _ptr(sc)))
         return dict(pvalue=pv, padj=padj, cooksCutoff=sc[0], filterThreshold=sc[1], filterTheta=sc[2], filterIndex=int(sc[3]))
 
     # -- setup ------------------------------------------------------------------------------

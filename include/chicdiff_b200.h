@@ -16,7 +16,7 @@
  *     :1573-1574, estimateDispersions + nbinomWaldTest                      -> cd_region_test
  *      1602-1603, 1643-1644, 1673-1674
  *     :1721,1730,1739  results(): Cook's cutoff, independent filtering, BH  -> cd_results_adjust,
- *                                                                              cd_results_resident
+ *                                                                              cd_results_resident, cd_results_device
  *   getFullRegionData(chicdiff.settings, RU, RUcontrol, suffix)            chicdiff.R:1460-1478
  *     supplies the per-row N / FullMean columns                            -> cd_set_sample_rows
  *
@@ -292,8 +292,16 @@ int cd_results_adjust(int64_t n, int S, int p, const double* baseMean, const dou
 /* The same results() step (chicdiff.R:1721,1730,1739) on the arrays the last successful cd_region_test of this
  * context left in device memory: two radix sorts and prefix counts on the GPU, only the 50-point lowess of the
  * filtering rule on the host.  pvalue_out / padj_out (n doubles each, host; either may be NULL) and scalars_out
- * as in cd_results_adjust.  Not for sharded contexts (the step is global): gather and use cd_results_adjust. */
+ * as in cd_results_adjust.  Not for sharded contexts (the step is global): gather and use cd_results_device or
+ * cd_results_adjust. */
 int cd_results_resident(cd_ctx* ctx, double* pvalue_out, double* padj_out, double* scalars_out);
+
+/* The same device routine on columns given by the caller: n host doubles each of baseMean, maxCooks (NULL = no Cook's
+ * filtering) and pvalue, n flag bytes (NULL = none carries CD_FLAG_COOKS_KEEP), and the design's S and p.  The columns are
+ * copied to the context's GPU; nothing of the context's last cd_region_test is read or changed.  For the gathered columns
+ * of a sharded run, or any columns results() should see.  Outputs as cd_results_resident; pvalue is not modified. */
+int cd_results_device(cd_ctx* ctx, int64_t n, int S, int p, const double* baseMean, const double* maxCooks,
+                      const uint8_t* flags, const double* pvalue, double* pvalue_out, double* padj_out, double* scalars_out);
 
 /* IHWcorrection(), "apply to test data" block (chicdiff.R:2038-2049), after R's ihw() has been trained on the control
  * set and the distance lookup learned (:1994-2033): minLogDist / maxLogDist / avWeights are the ngroups rows of

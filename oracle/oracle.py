@@ -224,7 +224,8 @@ def p_adjust_bh(p):
     ok = ~np.isnan(p)
     pv = p[ok]
     m = len(pv)
-    if m == 0:
+    if m <= 1:                                  # p.adjust: `if (n <= 1) return(p0)`, n = number of non-NA
+        out[ok] = pv
         return out
     o = np.argsort(-pv, kind="stable")          # decreasing
     ranks = np.arange(m, 0, -1)
@@ -236,15 +237,21 @@ def p_adjust_bh(p):
 
 
 def quantile7(x, probs):
+    """quantile(x, probs, type = 7) as quantile.default computes it: index <- 1 + (n - 1) * probs, lo <- floor(index),
+    hi <- ceiling(index), (1 - h) * x[lo] + h * x[hi] where index > lo and x[hi] != x[lo].  (The 4 * eps fuzz of
+    quantile.default belongs to types 4-9, not to type 7.)"""
     xs = np.sort(np.asarray(x, dtype=np.float64))
     n = len(xs)
-    h = (n - 1) * np.asarray(probs, dtype=np.float64)
-    lo = np.floor(h + 4 * np.finfo(float).eps).astype(np.int64)     # R's fuzz
-    lo = np.clip(lo, 0, n - 1)
-    hi = np.clip(lo + 1, 0, n - 1)
-    frac = h - lo
-    frac = np.where(np.abs(frac) < 4 * np.finfo(float).eps, 0.0, frac)
-    return xs[lo] + frac * (xs[hi] - xs[lo])
+    index = 1.0 + (n - 1) * np.asarray(probs, dtype=np.float64)
+    lo = np.floor(index)
+    hi = np.ceil(index)
+    h = index - lo
+    lo = lo.astype(np.int64) - 1
+    hi = hi.astype(np.int64) - 1
+    q = xs[lo]
+    with np.errstate(invalid="ignore"):
+        interp = (index > lo + 1) & (xs[hi] != q)
+        return np.where(interp, (1.0 - h) * q + h * xs[hi], q)
 
 
 def lowess(x, y, f=2.0 / 3.0, nsteps=3, delta=None):
@@ -345,7 +352,8 @@ def independent_filtering(base_mean, pvalue, alpha=0.1):
     """DESeq2 pvalueAdjustment (independentFiltering=TRUE, filter=baseMean).  Returns dict."""
     flt = np.asarray(base_mean, dtype=np.float64)
     p = np.asarray(pvalue, dtype=np.float64)
-    lower = np.mean(flt == 0)
+    # mean(filter == 0): R sums the logical in long double and rounds s / n to double
+    lower = float(np.longdouble(np.count_nonzero(flt == 0)) / np.longdouble(len(flt)))
     upper = .95 if lower < .95 else 1.0
     theta = np.linspace(lower, upper, 50)
     cut = quantile7(flt, theta)
