@@ -155,6 +155,30 @@ __global__ void count_flags_kernel(int64_t n, const uint8_t* __restrict__ flags,
     }
 }
 
+// layout of the small device scalar buffer ctx->scal (doubles)
+constexpr int kScalSf = 0;            // S size factors
+constexpr int kScalXim = 64;          // per fit: moments offset
+constexpr int kScalMed = 96;          // per fit: median of the log residuals
+constexpr int kScalMad = 128;         // per fit: 1.4826 x median absolute deviation
+constexpr int kScalDev = 160;         // per fit: total deviance
+constexpr int kScalTrend = 192;       // per fit: 8 doubles (coefficients, status, outer iterations, passes)
+constexpr int kScalSums = 384;        // per fit: S + 1 masked column sums of the normalisation factors
+constexpr int kScalSize = 1024;
+// layout of the pinned host scratch ctx->h_pinned (doubles)
+constexpr int kPinTrend = 0, kPinMad = 128, kPinErr = 144, kPinBad = 145, kPinDev = 160, kPinTrendIn = 200, kPinSf = 400;
+
+// layout of the device counter words ctx->counters (unsigned long long; word 11 is free)
+constexpr int kCntFlags = 0;          // 4: regions not all zero, gene-wise grid refits, MAP grid refits, GLMs not converged
+constexpr int kCntWait = 4;           // 3: SM cycles the trend fit waited for peers' sums, for its own slot, in its first pass
+constexpr int kCntBad = 7;            // a double: 1.0 when a count is NA or negative
+constexpr int kCntSelBar = 8;         // grid barrier of the medians (unsigned int)
+constexpr int kCntTrendBar = 9;       // grid barrier of the trend fit (unsigned int)
+constexpr int kCntErr = 10;           // non-zero when a peer-memory exchange gave up
+constexpr int kCntFitDispQueue = 12;  // 2: work-queue heads of the line search's two passes
+constexpr int kCntPark = 14;          // regions the line search parked
+constexpr int kCntWaldQueue = 15;     // work-queue head of the GLM fits
+constexpr int kCntSize = 16;
+
 }  // namespace
 
 struct cd_ctx {
@@ -491,8 +515,8 @@ int cd_comm_init(cd_ctx* ctx, int nranks, int rank, const char id[128])
     CD_CUDA(ctx, cudaSetDevice(ctx->device));
     CD_COMM(ctx, ctx->comm.init(nranks, rank, id));
     if (!ctx->counters.p) {
-        CD_CUDA(ctx, ctx->counters.ensure(16));
-        CD_CUDA(ctx, cudaMemset(ctx->counters.p, 0, 16 * sizeof(unsigned long long)));
+        CD_CUDA(ctx, ctx->counters.ensure(kCntSize));
+        CD_CUDA(ctx, cudaMemset(ctx->counters.p, 0, kCntSize * sizeof(unsigned long long)));
     }
     const std::string why = setup_p2p(ctx);
     if (!why.empty()) {
@@ -1195,18 +1219,6 @@ int cd_aggregate(cd_ctx* ctx, int32_t* K_out, double* fullmean_out)
 // ---------------------------------------------------------------------------------------------
 namespace {
 
-// layout of the small device scalar buffer ctx->scal (doubles)
-constexpr int kScalSf = 0;            // S size factors
-constexpr int kScalXim = 64;          // per fit: moments offset
-constexpr int kScalMed = 96;          // per fit: median of the log residuals
-constexpr int kScalMad = 128;         // per fit: 1.4826 x median absolute deviation
-constexpr int kScalDev = 160;         // per fit: total deviance
-constexpr int kScalTrend = 192;       // per fit: 8 doubles (coefficients, status, outer iterations, passes)
-constexpr int kScalSums = 384;        // per fit: S + 1 masked column sums of the normalisation factors
-constexpr int kScalSize = 1024;
-// layout of the pinned host scratch ctx->h_pinned (doubles)
-constexpr int kPinTrend = 0, kPinMad = 128, kPinErr = 144, kPinBad = 145, kPinDev = 160, kPinTrendIn = 200, kPinSf = 400;
-
 // R median() of the finite entries of B columns (column c at base + c*stride, n local values each, optionally
 // transformed to |x - center[c]|) over ALL ranks -> out_dev[c] = scale * median (exp'ed if do_exp): one cooperative
 // kernel; in a sharded run it all-reduces its 2048-bin counters through peer memory itself.
@@ -1218,7 +1230,7 @@ int medians(cd_ctx* ctx, const double* base, int64_t stride, int64_t n, int B, c
     CD_CUDA(ctx, ctx->sel_aux.ensure((size_t)kSelP2PMaxCols * 3));
     SelP2P pp{};
     pp.nranks = 1;
-    pp.err = ctx->counters.p + 10;
+    pp.err = ctx->counters.p + kCntErr;
     if (ctx->comm.active()) {
         pp.nranks = ctx->comm.nranks; pp.rank = ctx->comm.rank;
         pp.peers = ctx->sel_peers_dev.p; pp.mymail = ctx->sel_mail.p;
@@ -1226,7 +1238,7 @@ int medians(cd_ctx* ctx, const double* base, int64_t stride, int64_t n, int B, c
         ctx->sel_seq += kSelExchanges;
     }
     CD_LAUNCHN(ctx, 1, sel_launch_fused(n, B, base, stride, center_dev, out_dev, do_exp, scale, ctx->sel_state.p, ctx->sel_hist.p,
-                                        ctx->sel_aux.p, reinterpret_cast<unsigned int*>(ctx->counters.p + 8), pp, ctx->st));
+                                        ctx->sel_aux.p, reinterpret_cast<unsigned int*>(ctx->counters.p + kCntSelBar), pp, ctx->st));
     return CD_OK;
 }
 
@@ -1234,7 +1246,7 @@ int medians(cd_ctx* ctx, const double* base, int64_t stride, int64_t n, int B, c
 int check_peer_exchange(cd_ctx* ctx, unsigned long long err_word)
 {
     if (err_word == 0ull) return CD_OK;
-    cudaMemsetAsync(ctx->counters.p + 10, 0, sizeof(unsigned long long), ctx->st);
+    cudaMemsetAsync(ctx->counters.p + kCntErr, 0, sizeof(unsigned long long), ctx->st);
     return ctx->fail(CD_ECOMM, "peer-memory exchange timed out: another rank stopped before reaching the same step");
 }
 
@@ -1243,8 +1255,8 @@ int size_factors(cd_ctx* ctx, double* sf_host)
 {
     const int S = ctx->des.S;
     const int64_t n = ctx->n;
-    // counters[7] (zeroed at the start of every cd_region_test) is a double: 1.0 when a count is NA or negative
-    double* bad_dev = reinterpret_cast<double*>(ctx->counters.p + 7);
+    // zeroed at the start of every cd_region_test
+    double* bad_dev = reinterpret_cast<double*>(ctx->counters.p + kCntBad);
     CD_CUDA(ctx, ctx->g_LR.ensure((size_t)S * (size_t)n));
     CD_LAUNCHN(ctx, 1, launch_log_ratios(n, S, ctx->K.p, ctx->g_LR.p, bad_dev, ctx->st));
     int rc = medians(ctx, ctx->g_LR.p, n, n, S, nullptr, ctx->scal.p + kScalSf, 1, 1.0);
@@ -1252,7 +1264,7 @@ int size_factors(cd_ctx* ctx, double* sf_host)
     // every rank must refuse together, or the clean ones would wait for the others in the next collective
     CD_COMM(ctx, ctx->comm.allreduce_sum(bad_dev, 1, ctx->st));
     CD_CUDA(ctx, cudaMemcpyAsync(ctx->h_pinned + kPinSf, ctx->scal.p + kScalSf, sizeof(double) * S, cudaMemcpyDeviceToHost, ctx->st));
-    CD_CUDA(ctx, cudaMemcpyAsync(ctx->h_pinned + kPinErr, ctx->counters.p + 10, sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->st));
+    CD_CUDA(ctx, cudaMemcpyAsync(ctx->h_pinned + kPinErr, ctx->counters.p + kCntErr, sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->st));
     CD_CUDA(ctx, cudaMemcpyAsync(ctx->h_pinned + kPinBad, bad_dev, sizeof(double), cudaMemcpyDeviceToHost, ctx->st));
     CD_CUDA(ctx, cudaStreamSynchronize(ctx->st));
     unsigned long long errw;
@@ -1267,6 +1279,38 @@ int size_factors(cd_ctx* ctx, double* sf_host)
         if (std::isnan(sf_host[s]))
             return ctx->fail(CD_ENUMERIC, "every gene contains at least one zero, cannot compute log geometric means");
     }
+    return CD_OK;
+}
+
+// Timing section 2: one line search of a batch (gene-wise without a prior, MAP with one), then the count of its
+// posterior evaluations, which cd_last_search_counts reports per call.
+int timed_fit_disp(cd_ctx* ctx, int64_t nv, int64_t n, int S, int p, const CdDesign* des_dev, const int32_t* K,
+                   const double* prior_log_mean, const BatchScalars& prior_sigmasq, int32_t* iter)
+{
+    cudaStream_t st = ctx->st;
+    ctx->tm_begin(2);
+    CD_LAUNCHN(ctx, 2, launch_fit_disp(nv, n, S, p, des_dev, K, ctx->mu.p, ctx->start_log.p, prior_log_mean, prior_sigmasq,
+                                       ctx->log_alpha.p, iter, ctx->initial_lp.p, ctx->last_lp.p,
+                                       ctx->counters.p + kCntFitDispQueue, ctx->park, st));
+    ctx->tm_end();
+    if (ctx->n_eval_calls < 16 && nv > 0) {
+        count_evals_kernel<<<592, 256, 0, st>>>(nv, iter, ctx->eval_counts.p + ctx->n_eval_calls);
+        ctx->launches++;
+        ctx->eval_call_p[ctx->n_eval_calls] = p; ctx->eval_call_regions[ctx->n_eval_calls] = nv; ctx->n_eval_calls++;
+    }
+    return CD_OK;
+}
+
+// Timing section 4: the grid refit of the rows the preceding gene_post / map_post listed.
+int timed_grid_refit(cd_ctx* ctx, int64_t nv, int64_t n, int S, int p, const CdDesign* des_dev, const int32_t* K,
+                     const double* prior_mean_disp, const BatchScalars& prior_sigmasq, int grid_len, double* disp_out,
+                     double* dispersion_out, const uint8_t* flags, const double* dispGeneEst)
+{
+    ctx->tm_begin(4);
+    CD_LAUNCHN(ctx, 1, launch_fit_disp_grid(nv, n, S, p, des_dev, ctx->refit_count.p, ctx->refit_list.p, K, ctx->mu.p,
+                                            prior_mean_disp, prior_sigmasq, grid_len, disp_out, dispersion_out, flags,
+                                            dispGeneEst, ctx->st));
+    ctx->tm_end();
     return CD_OK;
 }
 
@@ -1295,7 +1339,7 @@ int run_batch(cd_ctx* ctx, const CdDesign& des, const CdDesign* des_dev, int G, 
     double* sums_dev = ctx->scal.p + kScalSums;
     double* xim_dev = ctx->scal.p + kScalXim;
     double* trend_dev = ctx->scal.p + kScalTrend;
-    unsigned long long* err_dev = ctx->counters.p + 10;
+    unsigned long long* err_dev = ctx->counters.p + kCntErr;
 
     BatchScalars th{};
     for (int g = 0; g < G; g++) th.v[g] = theta[g];
@@ -1314,21 +1358,12 @@ int run_batch(cd_ctx* ctx, const CdDesign& des, const CdDesign* des_dev, int G, 
     }
     BatchScalars none{};
     for (int g = 0; g < kMaxBatch; g++) none.v[g] = 1.0;
-    ctx->tm_begin(2);
-    CD_LAUNCHN(ctx, 2, launch_fit_disp(nv, n, S, p, des_dev, K, ctx->mu.p, ctx->start_log.p, nullptr, none, ctx->log_alpha.p,
-                                       ctx->dispGeneIter.p, ctx->initial_lp.p, ctx->last_lp.p, ctx->counters.p + 12, ctx->park, st));
-    ctx->tm_end();
-    if (ctx->n_eval_calls < 16 && nv > 0) {
-        count_evals_kernel<<<592, 256, 0, st>>>(nv, ctx->dispGeneIter.p, ctx->eval_counts.p + ctx->n_eval_calls);
-        ctx->launches++;
-        ctx->eval_call_p[ctx->n_eval_calls] = p; ctx->eval_call_regions[ctx->n_eval_calls] = nv; ctx->n_eval_calls++;
-    }
+    int rc = timed_fit_disp(ctx, nv, n, S, p, des_dev, K, nullptr, none, ctx->dispGeneIter.p);
+    if (rc != CD_OK) return rc;
     CD_LAUNCHN(ctx, 1, launch_gene_post(nv, S, ctx->alpha_init.p, ctx->log_alpha.p, ctx->dispGeneIter.p, ctx->initial_lp.p,
                                         ctx->last_lp.p, flags, dispGeneEst, ctx->refit_list.p, ctx->refit_count.p, st));
-    ctx->tm_begin(4);
-    CD_LAUNCHN(ctx, 1, launch_fit_disp_grid(nv, n, S, p, des_dev, ctx->refit_count.p, ctx->refit_list.p, K, ctx->mu.p, nullptr, none,
-                                            grid_len, dispGeneEst, nullptr, flags, dispGeneEst, st));
-    ctx->tm_end();
+    rc = timed_grid_refit(ctx, nv, n, S, p, des_dev, K, nullptr, none, grid_len, dispGeneEst, nullptr, flags, dispGeneEst);
+    if (rc != CD_OK) return rc;
     // trend + MAD of every fit over the regions of all ranks.  Nothing is gathered: the trend passes all-reduce 8 sums
     // per fit, the medians all-reduce histogram counters, both inside their kernels.  One host sync for both.
     ctx->tm_begin(5);
@@ -1346,13 +1381,13 @@ int run_batch(cd_ctx* ctx, const CdDesign& des, const CdDesign* des_dev, int G, 
         pp.peers = ctx->p2p_peers_dev.p; pp.mymail = ctx->p2p_mail.p;
         pp.epoch = ++ctx->p2p_epoch;
         pp.err = err_dev;
-        pp.wait_cycles = ctx->comm.active() ? ctx->counters.p + 4 : nullptr;
+        pp.wait_cycles = ctx->comm.active() ? ctx->counters.p + kCntWait : nullptr;
         CD_LAUNCHN(ctx, 1, launch_trend_fit(n, G, baseMean, dispGeneEst, flags, ctx->trend_xs.p, ctx->partial.p,
-                                            reinterpret_cast<unsigned int*>(ctx->counters.p + 9), trend_dev, pp, st));
+                                            reinterpret_cast<unsigned int*>(ctx->counters.p + kCntTrendBar), trend_dev, pp, st));
     }
     CD_LAUNCHN(ctx, 1, launch_trend_apply(nv, n, baseMean, dispGeneEst, flags, trend_dev, dispFit, ctx->g_resid.p,
                                           ctx->start_log.p, ctx->log_fit.p, st));
-    int rc = medians(ctx, ctx->g_resid.p, n, n, G, nullptr, ctx->scal.p + kScalMed, 0, 1.0);
+    rc = medians(ctx, ctx->g_resid.p, n, n, G, nullptr, ctx->scal.p + kScalMed, 0, 1.0);
     if (rc != CD_OK) return rc;
     rc = medians(ctx, ctx->g_resid.p, n, n, G, ctx->scal.p + kScalMed, ctx->scal.p + kScalMad, 0, 1.4826);
     if (rc != CD_OK) return rc;
@@ -1425,21 +1460,13 @@ int run_batch(cd_ctx* ctx, const CdDesign& des, const CdDesign* des_dev, int G, 
     ctx->trend_passes_batch = 0;
 
     // MAP
-    ctx->tm_begin(2);
-    CD_LAUNCHN(ctx, 2, launch_fit_disp(nv, n, S, p, des_dev, K, ctx->mu.p, ctx->start_log.p, ctx->log_fit.p, prior, ctx->log_alpha.p,
-                                       ctx->dispIter.p, ctx->initial_lp.p, ctx->last_lp.p, ctx->counters.p + 12, ctx->park, st));
-    ctx->tm_end();
-    if (ctx->n_eval_calls < 16 && nv > 0) {
-        count_evals_kernel<<<592, 256, 0, st>>>(nv, ctx->dispIter.p, ctx->eval_counts.p + ctx->n_eval_calls);
-        ctx->launches++;
-        ctx->eval_call_p[ctx->n_eval_calls] = p; ctx->eval_call_regions[ctx->n_eval_calls] = nv; ctx->n_eval_calls++;
-    }
+    rc = timed_fit_disp(ctx, nv, n, S, p, des_dev, K, ctx->log_fit.p, prior, ctx->dispIter.p);
+    if (rc != CD_OK) return rc;
     CD_LAUNCHN(ctx, 1, launch_map_post(nv, n, S, ctx->log_alpha.p, ctx->dispIter.p, dispGeneEst, dispFit, thr,
                                        flags, ctx->dispMAP.p, ctx->dispersion.p, ctx->refit_list.p, ctx->refit_count.p, st));
-    ctx->tm_begin(4);
-    CD_LAUNCHN(ctx, 1, launch_fit_disp_grid(nv, n, S, p, des_dev, ctx->refit_count.p, ctx->refit_list.p, K, ctx->mu.p, dispFit,
-                                            prior, grid_len, ctx->dispMAP.p, ctx->dispersion.p, flags, dispGeneEst, st));
-    ctx->tm_end();
+    rc = timed_grid_refit(ctx, nv, n, S, p, des_dev, K, dispFit, prior, grid_len, ctx->dispMAP.p, ctx->dispersion.p, flags,
+                          dispGeneEst);
+    if (rc != CD_OK) return rc;
     // NB GLM + Wald (final fit) / total deviance only (theta-grid fits)
     ctx->tm_begin(3);
     if (final_fit) {
@@ -1531,8 +1558,8 @@ int cd_region_test(cd_ctx* ctx, const cd_options* opt, cd_results* out)
     CD_CUDA(ctx, ctx->partial.ensure((size_t)kReduceBlocks * kMaxBatch * (CD_MAXS + 1)));
     CD_CUDA(ctx, ctx->scal.ensure(kScalSize));
     if (!ctx->counters.p) {
-        CD_CUDA(ctx, ctx->counters.ensure(16));
-        CD_CUDA(ctx, cudaMemsetAsync(ctx->counters.p, 0, 16 * sizeof(unsigned long long), st));
+        CD_CUDA(ctx, ctx->counters.ensure(kCntSize));
+        CD_CUDA(ctx, cudaMemsetAsync(ctx->counters.p, 0, kCntSize * sizeof(unsigned long long), st));
     }
     CD_CUDA(ctx, ctx->refit_count.ensure(1));
     CD_CUDA(ctx, ctx->wald_c.ensure((size_t)S * (size_t)n));
@@ -1545,7 +1572,7 @@ int cd_region_test(cd_ctx* ctx, const cd_options* opt, cd_results* out)
     }
     ctx->wald_ws.lfact = ctx->lfact.p;
     ctx->wald_ws.cmat = ctx->wald_c.p; ctx->wald_ws.beta0 = ctx->wald_b0.p; ctx->wald_ws.beta_nat = ctx->wald_b.p;
-    ctx->wald_ws.iter = ctx->wald_iter.p; ctx->wald_ws.work_counter = ctx->counters.p + 15;
+    ctx->wald_ws.iter = ctx->wald_iter.p; ctx->wald_ws.work_counter = ctx->counters.p + kCntWaldQueue;
     {
         const int64_t cap = nv / 4 + 4096;
         CD_CUDA(ctx, ctx->park_row.ensure((size_t)cap));
@@ -1555,12 +1582,12 @@ int cd_region_test(cd_ctx* ctx, const cd_options* opt, cd_results* out)
         pk.capacity = cap; pk.row = ctx->park_row.p;
         pk.a = ctx->park_d.p; pk.lp = pk.a + cap; pk.dlp = pk.lp + cap; pk.kappa = pk.dlp + cap; pk.lp0 = pk.kappa + cap;
         pk.iter = ctx->park_i.p; pk.iter_accept = pk.iter + cap;
-        pk.count = ctx->counters.p + 14;
+        pk.count = ctx->counters.p + kCntPark;
     }
 
     CD_CUDA(ctx, ctx->eval_counts.ensure(16));
     CD_CUDA(ctx, cudaMemsetAsync(ctx->eval_counts.p, 0, 16 * sizeof(unsigned long long), st));
-    CD_CUDA(ctx, cudaMemsetAsync(ctx->counters.p + 4, 0, 4 * sizeof(unsigned long long), st));     // [4..6] waits, [7] bad counts
+    CD_CUDA(ctx, cudaMemsetAsync(ctx->counters.p + kCntWait, 0, 4 * sizeof(unsigned long long), st));     // waits, bad counts
     ctx->n_eval_calls = 0;
     ctx->trend_passes = 0;
     CD_CUDA(ctx, cudaEventRecord(ctx->ev[2], st));
@@ -1603,16 +1630,16 @@ int cd_region_test(cd_ctx* ctx, const cd_options* opt, cd_results* out)
     out->trend_a0 = po.a0; out->trend_a1 = po.a1;
     out->varLogDispEsts = po.varLogDispEsts; out->dispPriorVar = po.dispPriorVar;
 
-    CD_CUDA(ctx, cudaMemsetAsync(ctx->counters.p, 0, 4 * sizeof(unsigned long long), st));
+    CD_CUDA(ctx, cudaMemsetAsync(ctx->counters.p + kCntFlags, 0, 4 * sizeof(unsigned long long), st));
     const uint8_t* flags = ctx->g_flags.p + ctx->g_off;
     if (n > 0) {
-        count_flags_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(n, flags, ctx->counters.p);
+        count_flags_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(n, flags, ctx->counters.p + kCntFlags);
         ctx->launches++;
     }
     unsigned long long hc[4] = {0, 0, 0, 0};
-    CD_CUDA(ctx, cudaMemcpyAsync(hc, ctx->counters.p, sizeof(hc), cudaMemcpyDeviceToHost, st));
+    CD_CUDA(ctx, cudaMemcpyAsync(hc, ctx->counters.p + kCntFlags, sizeof(hc), cudaMemcpyDeviceToHost, st));
     CD_CUDA(ctx, cudaMemcpyAsync(ctx->eval_counts_host, ctx->eval_counts.p, sizeof(ctx->eval_counts_host), cudaMemcpyDeviceToHost, st));
-    CD_CUDA(ctx, cudaMemcpyAsync(ctx->wait_host, ctx->counters.p + 4, sizeof(ctx->wait_host), cudaMemcpyDeviceToHost, st));
+    CD_CUDA(ctx, cudaMemcpyAsync(ctx->wait_host, ctx->counters.p + kCntWait, sizeof(ctx->wait_host), cudaMemcpyDeviceToHost, st));
     const size_t nn = (size_t)n;
     if ((rc = d2h(ctx, out->baseMean, ctx->g_baseMean.p + ctx->g_off, nn)) != CD_OK) return rc;
     if ((rc = d2h(ctx, out->baseVar, ctx->baseVar.p, nn)) != CD_OK) return rc;

@@ -190,16 +190,76 @@ static inline size_t fit_disp_smem_doubles(int S, int P, int threads)
     return (size_t)2 * S * threads + (size_t)(threads / 32) * 2 * fit_disp_block_doubles(S) + (size_t)S * P;
 }
 
+// the constants of DESeq2's fitDisp (DESeq2.cpp)
+constexpr double kSearchEpsilon = 1.0e-4, kSearchKappa0 = 1.0, kSearchTol = 1e-6;
+constexpr int kSearchMaxit = 100;
+
+// The scalar state of one region's line search: the current point a = log(alpha), the posterior and its derivative
+// there, the posterior at the start, the step factor and the trip counts.
+struct SearchState {
+    double a, lp, lp0, dlp, kappa;
+    int iter, iter_accept;
+};
+
+// one trip of fitDisp, first half: the next proposal, its step clamped to log(alpha) in [-30, 10]
+__device__ __forceinline__ double propose(SearchState& s)
+{
+    s.iter++;
+    const double a_propose = s.a + s.kappa * s.dlp;
+    if (a_propose < -30.0) s.kappa = (-30.0 - s.a) / s.dlp;
+    if (a_propose > 10.0) s.kappa = (10.0 - s.a) / s.dlp;
+    return s.a + s.kappa * s.dlp;
+}
+
+// second half: the Armijo test of the proposal x (posterior lpx, derivative dlpx), then accept and maybe stop, or shrink
+// the step; true when the search has finished.  min_log_alpha = log(kMinDisp / 10): the caller takes it once per thread
+// (the device log is not folded at compile time)
+__device__ __forceinline__ bool decide(SearchState& s, double x, double lpx, double dlpx, double min_log_alpha)
+{
+    bool finished = false;
+    const double theta_kappa = -1.0 * lpx;
+    const double theta_hat_kappa = -1.0 * s.lp - s.kappa * kSearchEpsilon * (s.dlp * s.dlp);
+    if (theta_kappa <= theta_hat_kappa) {
+        s.iter_accept++;
+        s.a = x;
+        const double change = lpx - s.lp;
+        if (change < kSearchTol) { s.lp = lpx; finished = true; }
+        else if (s.a < min_log_alpha) { finished = true; }
+        else {
+            s.lp = lpx;
+            s.dlp = dlpx;
+            s.kappa = fmin(s.kappa * 1.1, kSearchKappa0);
+            if (s.iter_accept % 5 == 0) s.kappa = s.kappa / 2.0;
+        }
+    } else {
+        s.kappa = s.kappa / 2.0;
+    }
+    if (s.iter >= kSearchMaxit) finished = true;
+    return finished;
+}
+
+__device__ __forceinline__ void park_store(const FitDispPark& park, unsigned long long slot, const SearchState& s)
+{
+    park.a[slot] = s.a; park.lp[slot] = s.lp; park.dlp[slot] = s.dlp; park.kappa[slot] = s.kappa; park.lp0[slot] = s.lp0;
+    park.iter[slot] = s.iter; park.iter_accept[slot] = s.iter_accept;
+}
+
+__device__ __forceinline__ SearchState park_load(const FitDispPark& park, int64_t w)
+{
+    SearchState s;
+    s.a = park.a[w]; s.lp = park.lp[w]; s.dlp = park.dlp[w]; s.kappa = park.kappa[w]; s.lp0 = park.lp0[w];
+    s.iter = park.iter[w]; s.iter_accept = park.iter_accept[w];
+    return s;
+}
+
 // Two passes.  ~2-3 % of the regions run the full 100 trips while the average is below 10; in a
 // single persistent pass such a region pulled near the end keeps its warp alive long after the
 // work queue is empty.  Pass 1 therefore parks every region that is still searching after
 // kFitDispTripCap trips (its scalar search state goes to the FitDispPark arrays); pass 2 resumes
 // all parked regions at once, one per lane, so the long searches overlap each other.
-#ifndef CD_FITDISP_MINBLOCKS
-#define CD_FITDISP_MINBLOCKS 4      /* <= 128 registers; measured in round 1: 5 blocks (<= 102) and 6 blocks (80) are not faster */
-#endif
-template <int P, bool RESUME, bool TABLOG>
-__global__ void __launch_bounds__(kFitDispThreads, CD_FITDISP_MINBLOCKS)
+constexpr int kFitDispMinBlocks = 4;    // <= 128 registers; measured in round 1: 5 blocks (<= 102) and 6 blocks (80) are not faster
+template <int P, bool RESUME>
+__global__ void __launch_bounds__(kFitDispThreads, kFitDispMinBlocks)
 fit_disp_kernel(int64_t n, int64_t n_fit, int S, const CdDesign* __restrict__ des, const int32_t* __restrict__ K,
                 const double* __restrict__ mu_g, const double* __restrict__ start_log,
                 const double* __restrict__ prior_log_mean, BatchScalars prior_inv_sigmasq_g,
@@ -209,15 +269,13 @@ fit_disp_kernel(int64_t n, int64_t n_fit, int S, const CdDesign* __restrict__ de
 {
     extern __shared__ __align__(16) double smem[];
     // logarithm table (16-byte aligned: one LDS.128 per logarithm); dynamic part: the lanes' columns, the warps' staged blocks, model matrix
-    __shared__ __align__(16) double tab[TABLOG ? 2 * kLogTabN : 2];
+    __shared__ __align__(16) double tab[2 * kLogTabN];
     const int stride = kFitDispThreads;
     double* ys = smem + threadIdx.x;
     double* mus = smem + (size_t)S * stride + threadIdx.x;
     const unsigned lane = threadIdx.x & 31u;
     const bool use_prior = (prior_log_mean != nullptr);
-    const double epsilon = 1.0e-4, kappa_0 = 1.0, tol = 1e-6;
     const double min_log_alpha = log(kMinDisp / 10.0);
-    const int maxit = 100;
     const double inv_n_fit = 1.0 / (double)n_fit;
     int64_t n_work = n;
     if (RESUME) {
@@ -227,8 +285,8 @@ fit_disp_kernel(int64_t n, int64_t n_fit, int S, const CdDesign* __restrict__ de
 
     bool active = false, exhausted = false, fresh = false;
     int64_t i = 0;
-    double a = 0.0, lp = 0.0, lp0 = 0.0, dlp = 0.0, kappa = kappa_0, prior_mean = 0.0, prior_sigmasq = 1.0;   // prior_sigmasq holds 1 / variance
-    int iter = 0, iter_accept = 0;
+    SearchState s{0.0, 0.0, 0.0, 0.0, kSearchKappa0, 0, 0};
+    double prior_mean = 0.0, prior_sigmasq = 1.0;      // prior_sigmasq holds 1 / variance
 
     // First pass: the inputs are staged per WARP.  A warp claims 32 consecutive regions with one atomic and its 32 lanes
     // copy their rows into a shared-memory block with cp.async (one coalesced request per row, all lanes active); two
@@ -240,7 +298,7 @@ fit_disp_kernel(int64_t n, int64_t n_fit, int S, const CdDesign* __restrict__ de
     double* blk0 = smem + (size_t)2 * S * stride + (size_t)(threadIdx.x >> 5) * 2 * blk_doubles;
     double* Xs = smem + (size_t)2 * S * stride + (size_t)(kFitDispThreads / 32) * 2 * blk_doubles;
     for (int k = threadIdx.x; k < S * P; k += blockDim.x) Xs[k] = des->X[k];
-    if (TABLOG) load_log_table(tab);
+    load_log_table(tab);
     const LogTab tabh = log_tab_handle(tab);
     __syncthreads();
 
@@ -321,7 +379,7 @@ fit_disp_kernel(int64_t n, int64_t n_fit, int S, const CdDesign* __restrict__ de
                         }
                         // the logarithms of the start value and of the prior mean were taken by the kernels that produced
                         // them (gene_init / trend_apply)
-                        a = a_start;
+                        s.a = a_start;
                         if (use_prior) {
                             prior_mean = mb[S * 32 + 32];
                             // the fit of virtual region i (no division of either kind on this path); eval_post multiplies
@@ -335,7 +393,7 @@ fit_disp_kernel(int64_t n, int64_t n_fit, int S, const CdDesign* __restrict__ de
                             prior_sigmasq = prior_inv_sigmasq_g.v[g];
                         }
                         active = true; fresh = true;
-                        iter = 0; iter_accept = 0; kappa = kappa_0;
+                        s.iter = 0; s.iter_accept = 0; s.kappa = kSearchKappa0;
                         want_now = false;
                     }
                 }
@@ -354,8 +412,7 @@ fit_disp_kernel(int64_t n, int64_t n_fit, int S, const CdDesign* __restrict__ de
                     exhausted = true;
                 } else {
                     i = park.row[w];
-                    a = park.a[w]; lp = park.lp[w]; dlp = park.dlp[w]; kappa = park.kappa[w]; lp0 = park.lp0[w];
-                    iter = park.iter[w]; iter_accept = park.iter_accept[w];
+                    s = park_load(park, w);
                     if (use_prior) {
                         prior_mean = prior_log_mean[i];
                         prior_sigmasq = prior_inv_sigmasq_g.v[(unsigned)i / (unsigned)n_fit];      // eval_post multiplies by the reciprocal
@@ -373,14 +430,8 @@ fit_disp_kernel(int64_t n, int64_t n_fit, int S, const CdDesign* __restrict__ de
             continue;
         }
         // ---- one posterior + derivative evaluation per active lane ----
-        double x = a;
-        if (active && !fresh) {
-            iter++;
-            const double a_propose = a + kappa * dlp;
-            if (a_propose < -30.0) kappa = (-30.0 - a) / dlp;
-            if (a_propose > 10.0) kappa = (10.0 - a) / dlp;
-            x = a + kappa * dlp;
-        }
+        double x = s.a;
+        if (active && !fresh) x = propose(s);
         // (explicit reconvergence: without it the branches above tail-merge into separate passes
         //  over the evaluation, which was measured at 13 of 32 lanes per issued instruction)
         __syncwarp();
@@ -388,48 +439,30 @@ fit_disp_kernel(int64_t n, int64_t n_fit, int S, const CdDesign* __restrict__ de
         // fitDisp evaluates the posterior at the proposal twice (Armijo test, then "lpnew") and, when
         // the proposal is accepted, the derivative at the same point; the arguments are the same
         // double, so one fused evaluation serves all three
-        if (active) eval_post<P, true, TABLOG>(x, ys, mus, stride, S, Xs, tabh, prior_mean, prior_sigmasq, use_prior, lpx, dlpx);
+        if (active) eval_post<P, true, true>(x, ys, mus, stride, S, Xs, tabh, prior_mean, prior_sigmasq, use_prior, lpx, dlpx);
         __syncwarp();
         // ---- decision ----
         bool finished = false;
         if (active) {
             if (fresh) {
-                lp = lp0 = lpx;
-                dlp = dlpx;
+                s.lp = s.lp0 = lpx;
+                s.dlp = dlpx;
                 fresh = false;
             } else {
-                const double theta_kappa = -1.0 * lpx;
-                const double theta_hat_kappa = -1.0 * lp - kappa * epsilon * (dlp * dlp);
-                if (theta_kappa <= theta_hat_kappa) {
-                    iter_accept++;
-                    a = x;
-                    const double change = lpx - lp;
-                    if (change < tol) { lp = lpx; finished = true; }
-                    else if (a < min_log_alpha) { finished = true; }
-                    else {
-                        lp = lpx;
-                        dlp = dlpx;
-                        kappa = fmin(kappa * 1.1, kappa_0);
-                        if (iter_accept % 5 == 0) kappa = kappa / 2.0;
-                    }
-                } else {
-                    kappa = kappa / 2.0;
-                }
-                if (iter >= maxit) finished = true;
+                finished = decide(s, x, lpx, dlpx, min_log_alpha);
             }
         }
         if (finished) {
-            log_alpha_out[i] = a;
-            iter_out[i] = iter;
-            initial_lp_out[i] = lp0;
-            last_lp_out[i] = lp;
+            log_alpha_out[i] = s.a;
+            iter_out[i] = s.iter;
+            initial_lp_out[i] = s.lp0;
+            last_lp_out[i] = s.lp;
             active = false;
-        } else if (!RESUME && active && iter >= kFitDispTripCap) {
+        } else if (!RESUME && active && s.iter >= kFitDispTripCap) {
             const unsigned long long slot = atomicAdd(park.count, 1ull);
             if (slot < (unsigned long long)park.capacity) {
                 park.row[slot] = i;
-                park.a[slot] = a; park.lp[slot] = lp; park.dlp[slot] = dlp; park.kappa[slot] = kappa; park.lp0[slot] = lp0;
-                park.iter[slot] = iter; park.iter_accept[slot] = iter_accept;
+                park_store(park, slot, s);
                 active = false;
             }                                   // park full: this lane simply keeps searching
         }
@@ -458,9 +491,7 @@ fit_disp_resume_tile_kernel(int64_t n, int64_t n_fit, int S, const CdDesign* __r
     const bool use_prior = (prior_log_mean != nullptr);
     const unsigned long long parked = *park.count;
     const int64_t n_work = (int64_t)(parked < (unsigned long long)park.capacity ? parked : (unsigned long long)park.capacity);
-    const double epsilon = 1.0e-4, kappa_0 = 1.0, tol = 1e-6;
     const double min_log_alpha = log(kMinDisp / 10.0);
-    const int maxit = 100;
     const bool has_sample = lane_g < S;
     double xrow[P];
 #pragma unroll
@@ -470,24 +501,17 @@ fit_disp_resume_tile_kernel(int64_t n, int64_t n_fit, int S, const CdDesign* __r
         const int64_t w = w0 + group;
         bool active = w < n_work;
         int64_t i = 0;
-        double a = 0.0, lp = 0.0, lp0 = 0.0, dlp = 1.0, kappa = kappa_0, prior_mean = 0.0, prior_sigmasq = 1.0, y = 0.0, mu = 1.0;
-        int iter = 0, iter_accept = 0;
+        SearchState s{0.0, 0.0, 0.0, 1.0, kSearchKappa0, 0, 0};
+        double prior_mean = 0.0, prior_sigmasq = 1.0, y = 0.0, mu = 1.0;
         if (active) {
             i = park.row[w];
-            a = park.a[w]; lp = park.lp[w]; dlp = park.dlp[w]; kappa = park.kappa[w]; lp0 = park.lp0[w];
-            iter = park.iter[w]; iter_accept = park.iter_accept[w];
+            s = park_load(park, w);
             if (use_prior) { prior_mean = prior_log_mean[i]; prior_sigmasq = prior_sigmasq_g.v[(unsigned)i / (unsigned)n_fit]; }
             if (has_sample) { y = (double)K[(int64_t)lane_g * n + i]; mu = mu_g[(int64_t)lane_g * n + i]; }
         }
         while (__any_sync(0xffffffffu, active)) {
-            double x = a;
-            if (active) {
-                iter++;
-                const double a_propose = a + kappa * dlp;
-                if (a_propose < -30.0) kappa = (-30.0 - a) / dlp;
-                if (a_propose > 10.0) kappa = (10.0 - a) / dlp;
-                x = a + kappa * dlp;
-            }
+            double x = s.a;
+            if (active) x = propose(s);
             // ---- this lane's replicate ----
             const double alpha = exp(x);
             const double r = rcp_pos(alpha);
@@ -536,41 +560,57 @@ fit_disp_resume_tile_kernel(int64_t n, int64_t n_fit, int S, const CdDesign* __r
                 dlpx += -1.0 * d / prior_sigmasq;
             }
             // ---- decision (identical in all lanes of the group) ----
-            if (active) {
-                bool finished = false;
-                const double theta_kappa = -1.0 * lpx;
-                const double theta_hat_kappa = -1.0 * lp - kappa * epsilon * (dlp * dlp);
-                if (theta_kappa <= theta_hat_kappa) {
-                    iter_accept++;
-                    a = x;
-                    const double change = lpx - lp;
-                    if (change < tol) { lp = lpx; finished = true; }
-                    else if (a < min_log_alpha) { finished = true; }
-                    else {
-                        lp = lpx;
-                        dlp = dlpx;
-                        kappa = fmin(kappa * 1.1, kappa_0);
-                        if (iter_accept % 5 == 0) kappa = kappa / 2.0;
-                    }
-                } else {
-                    kappa = kappa / 2.0;
-                }
-                if (iter >= maxit) finished = true;
-                if (finished) {
-                    if (lane_g == 0) { log_alpha_out[i] = a; iter_out[i] = iter; initial_lp_out[i] = lp0; last_lp_out[i] = lp; }
-                    active = false;
-                }
+            if (active && decide(s, x, lpx, dlpx, min_log_alpha)) {
+                if (lane_g == 0) { log_alpha_out[i] = s.a; iter_out[i] = s.iter; initial_lp_out[i] = s.lp0; last_lp_out[i] = s.lp; }
+                active = false;
             }
         }
     }
 }
 
-// CHICDIFF_B200_TABLE_LOG=0 selects the build of the line search that takes its logarithms with log_pos (fdlibm scheme)
-// instead of the shared-memory table; read at every launch so that a measurement script can switch between the two
-static bool table_log_enabled()
+// the two passes of launch_fit_disp for a design of P columns
+template <int P>
+static cudaError_t launch_fit_disp_p(int64_t n, int64_t n_fit, int S, const CdDesign* des, const int32_t* K, const double* mu,
+                                     const double* start_log, const double* prior_log_mean, const BatchScalars& prior_sigmasq,
+                                     double* log_alpha, int32_t* iter, double* initial_lp, double* last_lp,
+                                     unsigned long long* work_counter, const FitDispPark& park, cudaStream_t st)
 {
-    const char* e = getenv("CHICDIFF_B200_TABLE_LOG");
-    return !(e && e[0] == '0');
+    const int threads = kFitDispThreads;
+    const int64_t want = (n + threads - 1) / threads;
+    const size_t smem = fit_disp_smem_doubles(S, P, threads) * sizeof(double);
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    // Second pass: with few parked regions (small shards) the chain of up to 76 remaining trips is a latency
+    // problem -> sample-parallel tile kernel; with many it is a throughput problem -> one region per lane again.
+    const int G = S <= 8 ? 8 : (S <= 16 ? 16 : 32);
+    const bool tile = (double)n * 0.04 * G <= (double)sms * 1024.0;
+    BatchScalars prior_inv;                           // 1 / prior variance per fit (IEEE division, as the kernel's own would be)
+    for (int g = 0; g < kMaxBatch; g++) prior_inv.v[g] = 1.0 / prior_sigmasq.v[g];
+    // persistent grids: exactly the number of CTAs that are resident at once
+    int per_sm = 1;
+    cudaError_t e = cudaFuncSetAttribute(fit_disp_kernel<P, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fit_disp_kernel<P, false>, threads, smem);
+    if (e != cudaSuccess) return e;
+    const int64_t resident = (int64_t)sms * (per_sm > 0 ? per_sm : 1);
+    const int blocks = (int)(want < resident ? want : resident);
+    fit_disp_kernel<P, false><<<blocks, threads, smem, st>>>(n, n_fit, S, des, K, mu, start_log, prior_log_mean, prior_inv,
+                                                             log_alpha, iter, initial_lp, last_lp, work_counter, park);
+    if (tile) {
+        auto* tile_kernel = G == 8 ? fit_disp_resume_tile_kernel<P, 8>
+                                   : (G == 16 ? fit_disp_resume_tile_kernel<P, 16> : fit_disp_resume_tile_kernel<P, 32>);
+        tile_kernel<<<sms * 8, 128, 0, st>>>(n, n_fit, S, des, K, mu, prior_log_mean, prior_sigmasq, log_alpha, iter,
+                                             initial_lp, last_lp, park);
+    } else {
+        e = cudaFuncSetAttribute(fit_disp_kernel<P, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+        const int64_t want2 = (park.capacity + threads - 1) / threads;
+        const int blocks2 = (int)(want2 < resident ? want2 : resident);
+        fit_disp_kernel<P, true><<<blocks2 > 0 ? blocks2 : 1, threads, smem, st>>>(n, n_fit, S, des, K, mu, start_log,
+            prior_log_mean, prior_inv, log_alpha, iter, initial_lp, last_lp, work_counter + 1, park);
+    }
+    return cudaGetLastError();
 }
 
 cudaError_t launch_fit_disp(int64_t n, int64_t n_fit, int S, int p, const CdDesign* des, const int32_t* K, const double* mu,
@@ -584,63 +624,16 @@ cudaError_t launch_fit_disp(int64_t n, int64_t n_fit, int S, int p, const CdDesi
     if (e != cudaSuccess) return e;
     e = cudaMemsetAsync(park.count, 0, sizeof(unsigned long long), st);
     if (e != cudaSuccess) return e;
-    const int threads = kFitDispThreads;
-    const int64_t want = (n + threads - 1) / threads;
-    const size_t smem = fit_disp_smem_doubles(S, p, threads) * sizeof(double);
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    // Second pass: with few parked regions (small shards) the chain of up to 76 remaining trips is a latency
-    // problem -> sample-parallel tile kernel; with many it is a throughput problem -> one region per lane again.
-    const int G = S <= 8 ? 8 : (S <= 16 ? 16 : 32);
-    const bool tile = (double)n * 0.04 * G <= (double)sms * 1024.0;
-    const bool tl = table_log_enabled();
-    BatchScalars prior_inv;                           // 1 / prior variance per fit (IEEE division, as the kernel's own would be)
-    for (int g = 0; g < kMaxBatch; g++) prior_inv.v[g] = 1.0 / prior_sigmasq.v[g];
-    // persistent grids: exactly the number of CTAs that are resident at once
-#define CD_LAUNCH_T(P_, TL_)                                                                                   \
-    {                                                                                                          \
-        int per_sm = 1;                                                                                        \
-        e = cudaFuncSetAttribute(fit_disp_kernel<P_, false, TL_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-        if (e != cudaSuccess) return e;                                                                        \
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fit_disp_kernel<P_, false, TL_>, threads, smem); \
-        if (e != cudaSuccess) return e;                                                                        \
-        const int64_t resident = (int64_t)sms * (per_sm > 0 ? per_sm : 1);                                     \
-        const int blocks = (int)(want < resident ? want : resident);                                           \
-        fit_disp_kernel<P_, false, TL_><<<blocks, threads, smem, st>>>(n, n_fit, S, des, K, mu, start_log,     \
-            prior_log_mean, prior_inv, log_alpha, iter, initial_lp, last_lp, work_counter, park);              \
-        if (tile) {                                                                                            \
-            const int blocks2 = sms * 8;                                                                       \
-            if (S <= 8)                                                                                        \
-                fit_disp_resume_tile_kernel<P_, 8><<<blocks2, 128, 0, st>>>(n, n_fit, S, des, K, mu, prior_log_mean, \
-                    prior_sigmasq, log_alpha, iter, initial_lp, last_lp, park);                                \
-            else if (S <= 16)                                                                                  \
-                fit_disp_resume_tile_kernel<P_, 16><<<blocks2, 128, 0, st>>>(n, n_fit, S, des, K, mu, prior_log_mean, \
-                    prior_sigmasq, log_alpha, iter, initial_lp, last_lp, park);                                \
-            else                                                                                               \
-                fit_disp_resume_tile_kernel<P_, 32><<<blocks2, 128, 0, st>>>(n, n_fit, S, des, K, mu, prior_log_mean, \
-                    prior_sigmasq, log_alpha, iter, initial_lp, last_lp, park);                                \
-        } else {                                                                                               \
-            e = cudaFuncSetAttribute(fit_disp_kernel<P_, true, TL_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-            if (e != cudaSuccess) return e;                                                                    \
-            const int64_t want2 = (park.capacity + threads - 1) / threads;                                     \
-            const int blocks2 = (int)(want2 < resident ? want2 : resident);                                    \
-            fit_disp_kernel<P_, true, TL_><<<blocks2 > 0 ? blocks2 : 1, threads, smem, st>>>(n, n_fit, S, des, K, mu, \
-                start_log, prior_log_mean, prior_inv, log_alpha, iter, initial_lp, last_lp,                    \
-                work_counter + 1, park);                                                                       \
-        }                                                                                                      \
-    }
-#define CD_LAUNCH(P_) { if (tl) CD_LAUNCH_T(P_, true) else CD_LAUNCH_T(P_, false) }
+    decltype(&launch_fit_disp_p<1>) launch;
     switch (p) {
-        case 1: CD_LAUNCH(1); break;
-        case 2: CD_LAUNCH(2); break;
-        case 3: CD_LAUNCH(3); break;
-        case 4: CD_LAUNCH(4); break;
+        case 1: launch = launch_fit_disp_p<1>; break;
+        case 2: launch = launch_fit_disp_p<2>; break;
+        case 3: launch = launch_fit_disp_p<3>; break;
+        case 4: launch = launch_fit_disp_p<4>; break;
         default: return cudaErrorInvalidValue;
     }
-#undef CD_LAUNCH
-#undef CD_LAUNCH_T
-    return cudaGetLastError();
+    return launch(n, n_fit, S, des, K, mu, start_log, prior_log_mean, prior_sigmasq, log_alpha, iter, initial_lp, last_lp,
+                  work_counter, park, st);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -662,7 +655,7 @@ gene_post_kernel(int64_t n, int S, const double* __restrict__ alpha_init, const 
     const double l0 = initial_lp[i];
     if (last_lp[i] < l0 + fabs(l0) / 1e6) { disp = alpha_init[i]; f |= CD_FLAG_GENE_NOINCREASE; }
     const int it = iter[i];
-    const bool conv = (it < 100) && (it != 1);
+    const bool conv = (it < kSearchMaxit) && (it != 1);
     if (!conv && disp > kMinDisp * 10.0) {
         f |= CD_FLAG_GENE_GRID;
         const int32_t slot = atomicAdd(refit_count, 1);
@@ -695,7 +688,7 @@ map_post_kernel(int64_t n, int64_t n_fit, int S, const double* __restrict__ log_
     uint8_t f = flags[i];
     if (f & CD_FLAG_ALLZERO) { dispMAP[i] = NAN; dispersion[i] = NAN; return; }
     const double maxDisp = fmax(10.0, (double)S);
-    if (!(iter[i] < 100)) {
+    if (!(iter[i] < kSearchMaxit)) {
         f |= CD_FLAG_MAP_GRID;
         const int32_t slot = atomicAdd(refit_count, 1);
         refit_list[slot] = (int32_t)i;

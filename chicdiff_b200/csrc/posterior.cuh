@@ -28,7 +28,8 @@ namespace cd {
 //     f^3 <= 1e-6 and higher: <= 3e-17 absolute), which makes them instruction immediates instead of constant loads;
 //   * p = 1 and p = 2 (every fit of the default pipeline) use the closed-form determinant and inverse of X'WX with
 //     one Newton reciprocal and one logarithm; p = 3, 4 keep the packed Cholesky;
-//   * TABLOG = true takes every logarithm with log_pos_v2 (table in shared memory, no reciprocal); false with log_pos.
+//   * TABLOG = true takes every logarithm with log_pos_v2 (table in shared memory, no reciprocal): the line search
+//     (fit_disp_kernel); false with log_pos: the grid refit (fit_disp_grid_kernel), which has no table.
 // ---------------------------------------------------------------------------------------
 struct GammaParts { double st, dgs, num, den; };      // st: Stirling part of lgamma; dgs: series part of digamma
 

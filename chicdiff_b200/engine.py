@@ -9,7 +9,8 @@ import os
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# (CHICDIFF_B200_LIB: development hook of scripts/fit_variants.py to time alternative builds of the same library)
+# (CHICDIFF_B200_LIB: development hook to load another build of the same library, e.g. to compare two builds'
+# outputs and timings; scripts/results_resident_check.py uses it)
 _LIB_PATH = os.environ.get("CHICDIFF_B200_LIB") or os.path.join(_HERE, "libchicdiff_b200.so")
 _lib = None
 

@@ -54,7 +54,7 @@ def data(name, p4=False, **kw):
 
 
 def oracle(key, d, prior=None, prior_grid=None, **kw):
-    """the oracle's run of a case (kept for the table-log rerun of the same case)"""
+    """the oracle's run of a case, once per session"""
     if key not in _ORACLE:
         K, FM = O.aggregate(d.row_off, d.N_rows, d.FM_rows)
         _ORACLE[key] = parity.oracle_region_test(K, FM, d.X, prior, prior_grid, **kw)
@@ -164,24 +164,6 @@ def test_lane_resume_with_prior(case):
     ro = oracle((case, 1e3), d, prior=1e3, theta=0.5)
     assert lane_resume(d.n, d.S)
     assert int((ro["dispIter"] > TRIP_CAP).sum()) > 100 and map_grid(ro) > 100
-    run(d, ro, prior=1e3, theta=0.5)
-
-
-# ---- the line search with log_pos instead of the logarithm table -----------------------------------------------------
-
-@pytest.mark.parametrize("case", ["map_grid", "lane_resume"])
-def test_without_the_log_table(case, monkeypatch):
-    """CHICDIFF_B200_TABLE_LOG=0 (read at every launch) selects the build of the line search that takes its logarithms
-    with log_pos; it must pass the same gate"""
-    monkeypatch.setenv("CHICDIFF_B200_TABLE_LOG", "0")
-    if case == "map_grid":
-        d = data("c1")
-        ro = oracle(("c1", 1e3), d, prior=1e3, theta=0.5)
-        assert map_grid(ro) > 5000
-    else:
-        d = data("c3", n_regions=140000, reps=(16, 16))
-        ro = oracle(("16v16_p2", 1e3), d, prior=1e3, theta=0.5)
-        assert lane_resume(d.n, d.S)
     run(d, ro, prior=1e3, theta=0.5)
 
 
